@@ -2,9 +2,10 @@
 """bench.py — BASELINE.json's headline metric on its config: Mrays/s incoherent closest-hit,
 synthetic 1M-triangle random-soup mesh, 16M-ray batch of diffuse bounce rays (config 3).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
-One "step" = one pass of the closest-hit path over one 16,777,216-ray batch.
+One "step" = one pass of the closest-hit path over one 16,777,216-ray batch; the any-hit, host-buffer and
+path-traced legs time K passes (frames) of their own as well.
   value  : rays already resident in HBM, K launches timed with CUDA events on the launching
            stream (rrt_intersect_device), max over ranks.
   e2e    : the same batch through the host-buffer C-ABI call a Rust `impl Primitive` binds
@@ -13,6 +14,10 @@ One "step" = one pass of the closest-hit path over one 16,777,216-ray batch.
            its own 16M-ray batch (weak scaling, no data-path collective).
 `--impl reference` times the CPU restatement of the reference's own BVH path (oracle/, all host
 threads) on bounded samples of the same workload — the Rust reference cannot be built here.
+`--dump-outputs DIR` writes, on rank 0, what the last timed step of each leg returned, as DIR/<name>.npy:
+a fixed, seeded sample of the rays (hits: prim_id with -1 for a miss, t, u, v; any-hit: occluded) and of
+the pixels of each path-traced frame (RGB).  The inputs are seeded, so two builds can be compared array
+for array (the films to rounding: they are summed with f64 atomics).
 """
 from __future__ import annotations
 
@@ -41,6 +46,29 @@ UNIT = "Mrays/s"
 NV_C3 = 122.98
 NT_C3 = 20.02
 BYTES_PER_RAY = 32 + 16 + 32 * NV_C3 + 36 * NT_C3
+# --dump-outputs: rays and pixels kept per array (38 MiB of .npy files in all)
+DUMP_RAYS = 1 << 19
+DUMP_PIXELS = 1 << 18
+DUMP_SEED = 20261020
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def sample_rows(n, k):
+    """The same min(n, k) row indices of an n-row output on every run, increasing."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+
+
+def write_dump(directory, arrays):
+    out = Path(directory)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(out / f"{name}.npy", a)
 
 
 def workload_config(n_gpus, n_rays=N_RAYS):
@@ -193,10 +221,11 @@ PT_CONFIGS = {
 }
 
 
-def path_traced(args, ctx, rank, world, local_rank, barrier, config):
+def path_traced(args, ctx, rank, world, local_rank, barrier, config, dump):
     """Second half of BASELINE.json's metric: one path-traced frame, its 16x16 sample tiles dealt
     t % world == rank over the ranks (scene replicated), films summed onto rank 0 over NCCL.
-    Strong scaling: the frame is fixed, value = camera samples of the whole frame / max-over-ranks time."""
+    Strong scaling: the frame is fixed, value = camera samples of the whole frame / max-over-ranks time.
+    A sample of the last timed frame's pixels goes into `dump` unless it is None."""
     import tempfile
     import torch
     import torch.distributed as dist
@@ -211,8 +240,7 @@ def path_traced(args, ctx, rank, world, local_rank, barrier, config):
     else:
         keep, r = synth.scene_c5_api(ctx, commit=(lambda a: parallel.commit_replicated(a, 4)) if world > 1 else None)
     setup_s = time.perf_counter() - t_setup
-    # config 5 is 2.1 G camera samples: one timed frame
-    frames = max(1, min(args.steps, 3)) if config == "c4" else 1
+    frames = args.steps
 
     def frame():
         r.clear()
@@ -247,6 +275,10 @@ def path_traced(args, ctx, rank, world, local_rank, barrier, config):
     out = None
     if rank == 0:
         img = r.film()
+        if dump is not None:
+            pix = sample_rows(img.shape[0] * img.shape[1], DUMP_PIXELS)
+            dump[f"path_{config}_pixel_index"] = pix.astype(np.float64)
+            dump[f"path_{config}_rgb"] = img.reshape(-1, 3)[pix]
         out = {
             "metric": "Msamples/s path-traced", "unit": "Msamples/s", "value": samples / (dt / frames) / 1e6,
             "ms_per_frame": dt / frames * 1e3, "frames": frames, "warmup_frame_ms": warm_s * 1e3, "n_gpus": world, "scaling": "strong",
@@ -333,10 +365,17 @@ def main():
     ap.add_argument("--path-config", default="both", choices=["both", "c4", "c5", "none"],
                     help="second half of the metric: path-traced Msamples/s on config 4 (1080p, 64 spp) and config 5 "
                          "(4K, 256 spp, the multi-GPU configuration)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of what the last timed step of each leg computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs: use it with --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    dump = {} if args.dump_outputs and rank == 0 else None
     if args.impl == "reference":
         run_reference(args, rank, world)
         return 0
@@ -399,6 +438,14 @@ def main():
     total_ms_max = float(t.item())
     value = n_rays * world * args.steps / (total_ms_max * 1e-3) / 1e6
     n_hit = int((d_hits.view(torch.int64)[0::4] & 0xFFFFFFFF != 0xFFFFFFFF).sum().item())
+    if dump is not None:
+        rows = sample_rows(n_rays, DUMP_RAYS)
+        d_rows = torch.from_numpy(rows).cuda()
+        h = d_hits.view(n_rays, 4)[d_rows].cpu().numpy().view(HIT_DTYPE).reshape(-1)
+        dump["ray_index"] = rows.astype(np.float64)
+        dump["closest_hit_prim_id"] = np.where(h["prim_id"] == 0xFFFFFFFF, -1.0, h["prim_id"].astype(np.float64))
+        for f in ("t", "u", "v"):
+            dump[f"closest_hit_{f}"] = np.ascontiguousarray(h[f])
 
     # ---- the other half of a1/a2: any-hit (BVHAccel::intersect_p) on the same batch, device resident ----
     d_occ = torch.empty(n_rays, dtype=torch.uint8, device="cuda")
@@ -418,6 +465,8 @@ def main():
     n_occ = int(d_occ.sum(dtype=torch.int64).item())
     if n_occ != n_hit:
         raise SystemExit(f"bench.py: any-hit and closest-hit disagree on which rays hit ({n_occ} vs {n_hit})")
+    if dump is not None:
+        dump["any_hit_occluded"] = d_occ[d_rows].float().cpu().numpy()
     del d_occ
 
     # ---- end to end: host buffers through rrt_intersect (H2D + kernel + D2H per step) ----
@@ -443,9 +492,11 @@ def main():
     del agg
     pt = pt5 = None
     if args.path_config in ("both", "c4"):
-        pt = path_traced(args, ctx, rank, world, local_rank, barrier, "c4")
+        pt = path_traced(args, ctx, rank, world, local_rank, barrier, "c4", dump)
     if args.path_config in ("both", "c5"):
-        pt5 = path_traced(args, ctx, rank, world, local_rank, barrier, "c5")
+        pt5 = path_traced(args, ctx, rank, world, local_rank, barrier, "c5", dump)
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
 
     if rank == 0:
         peak, peak_src = measured_peak()

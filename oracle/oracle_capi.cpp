@@ -70,7 +70,6 @@ void* orc_scene_new(uint32_t quirk_mask) {
     s->geom.q = quirks_from_mask(quirk_mask);
     return s;
 }
-void orc_scene_free(void* s) { delete (Scene*)s; }
 
 // create_triangle_mesh (triangle.rs:131-165).  Index arrays are 0-based; pass n=0 / null
 // for absent normals / uvs.  Returns the mesh index.
@@ -440,6 +439,16 @@ RenderSetup& setup_of(void* s) {
 
 extern "C" {
 
+// Drops the scene's render setup too: a later scene may be allocated at the same address.
+void orc_scene_free(void* s) {
+    for (size_t i = 0; i < g_setups.size(); ++i)
+        if (g_setups[i].first == s) {
+            g_setups.erase(g_setups.begin() + i);
+            break;
+        }
+    delete (Scene*)s;
+}
+
 // Debug ray log (rt_render.hpp raylog()): begin, render single-threaded, then take the records.
 void orc_raylog_begin() {
     static std::vector<double> store;
@@ -623,11 +632,6 @@ void orc_texture_probe(uint32_t n, const double* table, const double* uv2, const
     tex_eval_all(rs.textures, q, vals);
     for (uint32_t i = 0; i < n && i < (uint32_t)kMaxTextures; ++i)
         for (int c = 0; c < 3; ++c) out[3 * i + c] = vals[i].c[c];
-    for (size_t i = 0; i < g_setups.size(); ++i)
-        if (g_setups[i].first == tmp) {
-            g_setups.erase(g_setups.begin() + i);
-            break;
-        }
     orc_scene_free(tmp);
 }
 // compute_differentials probe: in = p n dpdu dpdv rx_o rx_d ry_o ry_d (3 doubles each); out = dpdx dpdy dudx dvdx dudy dvdy
@@ -707,11 +711,6 @@ void orc_area_light_probe(const double* row80, const double* ref_p3, const doubl
     Rgb L = sc.area_sample_li(rs.light_specs[0], V3(ref_p3[0], ref_p3[1], ref_p3[2]), P2(u2[0], u2[1]), &wi, &pdf, &p1);
     const double o[10] = {wi.x, wi.y, wi.z, pdf, p1.x, p1.y, p1.z, L.c[0], L.c[1], L.c[2]};
     std::memcpy(out10, o, sizeof(o));
-    for (size_t i = 0; i < g_setups.size(); ++i)
-        if (g_setups[i].first == tmp) {
-            g_setups.erase(g_setups.begin() + i);
-            break;
-        }
     orc_scene_free(tmp);
 }
 

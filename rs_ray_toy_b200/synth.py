@@ -240,8 +240,8 @@ def scene_c1_as_shipped(directory):
     """Config 1 exactly as the reference ships it (samples/scene.json): the same geometry, lights, film and camera as
     scene_c1, plus what scene_c1 leaves out — the unreferenced WindyTexture / ImageTexture("s_01.png") declarations,
     the `Debug` material, `Integrator {Debug, light_strategy all}` and `Sampler {StratifiedSampler}` (4 x 4, jittered,
-    4 sampled dimensions by default).  tests/test_reference_image.py checks this dict against the reference's file
-    when /root/reference is present.  s_01.png is NOT written: no material names that texture."""
+    4 sampled dimensions by default).  tests/test_reference_image.py checks this dict against a stored copy of the
+    reference's file (tests/golden/scene_c1_as_shipped.json).  s_01.png is NOT written: no material names that texture."""
     import json
     import os
     cfg = json.loads(open(scene_c1(directory)).read())

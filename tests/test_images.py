@@ -91,6 +91,16 @@ def test_mipmap_equals_the_oracles(tmp_path, w, h, tri, wrap):
         assert len(np.unique(got[:, 3])) > 100
 
 
+def test_a_new_oracle_scene_holds_no_images_of_a_freed_one():
+    """The oracle keys a scene's images by its address, which a scene made after a free may reuse."""
+    Lo, _ = _libs()
+    img = np.zeros((140, 300, 3), dtype=np.uint8)
+    for _ in range(3):
+        sc = Lo.orc_scene_new(0)
+        assert [Lo.orc_add_image(sc, 300, 140, img.ctypes.data, 0, 8.0, 0) for _ in range(3)] == [0, 1, 2]
+        Lo.orc_scene_free(sc)
+
+
 def test_tiny_images_are_refused():
     """An 8 x 8 level indexes outside its BlockedArray: the reference panics at load (memory.rs:76-85)."""
     _, Ld = _libs()

@@ -1,5 +1,6 @@
 import sys, time
-sys.path.insert(0, '/root/repo')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 from rs_ray_toy_b200 import capi, synth
 from rs_ray_toy_b200.aggregate import Context, soup_aggregate
 ctx = Context(0)
