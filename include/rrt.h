@@ -57,6 +57,26 @@ typedef struct rrt_hit {
     double v;
 } rrt_hit;
 
+/* Compact records for callers that hold their rays in fp32 (rrt_intersect_f32 and relatives below).  The aggregate
+ * still decides in f64: every float is promoted exactly to double on the device (`time` = 0, which the aggregate never
+ * reads: its transforms are static), the f64 walk runs unchanged, and each f64 result field is rounded to nearest
+ * (__double2float_rn) on the way out.  So a call on rrt_ray_f32 records returns bit for bit the rrt_intersect answer
+ * on the promoted rays, rounded.  t_max may be +inf.  32 bytes: two 16-byte loads per ray.                         */
+typedef struct rrt_ray_f32 {
+    float o[3];
+    float t_max;
+    float d[3];
+    uint32_t reserved; /* ignored */
+} rrt_ray_f32;
+/* rrt_hit with t, u, v rounded to nearest fp32; prim_id copied unchanged (RRT_NO_HIT on a miss, when t, u, v are the
+ * rounded values the f64 record carries).  16 bytes.                                                            */
+typedef struct rrt_hit_f32 {
+    uint32_t prim_id;
+    float t;
+    float u;
+    float v;
+} rrt_hit_f32;
+
 /* BVHSplitMethod (bvh.rs:111-114) plus the parity tier (SURVEY.md §8c).                         */
 typedef enum rrt_build_flags {
     RRT_BUILD_FAST = 0,    /* Tier F: own SAH tree, true closest hit, ties -> lowest prim id     */
@@ -145,6 +165,22 @@ int rrt_intersect_p_device(const rrt_scene* scene, uint64_t n, const rrt_ray* d_
  * binds (INTEGRATION.md).                                                                       */
 int rrt_intersect(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, rrt_hit* hits);
 int rrt_intersect_p(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, uint8_t* occluded);
+
+/* The same four calls on fp32 rays (rrt_ray_f32, 32 B) and compact hits (rrt_hit_f32, 16 B): Scene::intersect /
+ * intersect_p (scene.rs:69-80, bvh.rs:123-236) for callers whose rays are fp32 already, at half the link bytes per
+ * ray up and down.  Errors, limits and threading are those of the f64 call each one mirrors.
+ * Host buffers: the same chunked pipeline as rrt_intersect; the first fp32 call on a context adds one staging buffer
+ * of 32 MiB to each of its four pipeline slots (128 MiB of device memory, kept until rrt_destroy).                   */
+int rrt_intersect_f32(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* rays, rrt_hit_f32* hits);
+int rrt_intersect_p_f32(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* rays, uint8_t* occluded);
+/* Device buffers, asynchronous on `cuda_stream`.  The promoted f64 rays and the f64 hits live in scratch memory the
+ * scene keeps per calling stream: 96 bytes per ray for rrt_intersect_f32_device, 64 for rrt_intersect_p_f32_device,
+ * grown to the largest batch seen on that stream and freed by rrt_scene_destroy.  Past eight streams the scratch of
+ * the first one is shared, each call ordered after the last one that used it (as the tree walk's own workspaces).  */
+int rrt_intersect_f32_device(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, rrt_hit_f32* d_hits,
+                             void* cuda_stream);
+int rrt_intersect_p_f32_device(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, uint8_t* d_occluded,
+                               void* cuda_stream);
 
 /* ---- the render loop ------------------------------------------------------------------------
  * What deploy_render builds and runs (renderprocess.rs:92-105): make_scene + make_integrator,

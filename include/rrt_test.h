@@ -73,6 +73,11 @@ int rrt_stratified_host_probe(uint64_t seed, int64_t xres, int64_t px, int64_t p
  * lookups of csrc/mipmap_core.h run on the host: lookup_d -> out6[0..2], lookup_w(st, width = dstdx[0]) -> out6[3..5];
  * info = levels, then (u_res, v_res) per level.  rrt_envlight_host_probe: InfiniteAreaLight::new's distribution, then per
  * query (ref point[3], u[2], w[3]): sample_li -> Li[3], wi[3], pdf; pdf_li(w); le(w)[3]; p1.x.                        */
+/* Host-only probe of the fp32 record format (csrc/rays_f32.cuh, the conversions the streaming kernels around the walk
+ * run): promoted[i] = rays[i] as the rrt_ray the walk sees, compact[i] = hits[i] as the rrt_hit_f32 the caller gets. */
+int rrt_rays_f32_host_probe(uint64_t n_rays, const rrt_ray_f32* rays, rrt_ray* promoted, uint64_t n_hits, const rrt_hit* hits,
+                            rrt_hit_f32* compact);
+
 int rrt_png_host_probe(const char* path, uint32_t* width, uint32_t* height, uint8_t* rgb8, uint64_t capacity);
 int rrt_mipmap_host_probe(uint32_t width, uint32_t height, const uint8_t* rgb8, int trilinear, double max_aniso, uint32_t wrap,
                           uint64_t n, const double* q6, double* out6, uint64_t info[32]);

@@ -18,6 +18,10 @@ from . import capi
 RAY_DTYPE = np.dtype([("o", "<f8", 3), ("d", "<f8", 3), ("t_max", "<f8"), ("time", "<f8")])  # rrt_ray, 64 B
 HIT_DTYPE = np.dtype([("prim_id", "<u4"), ("reserved", "<u4"), ("t", "<f8"), ("u", "<f8"), ("v", "<f8")])  # rrt_hit, 32 B
 assert RAY_DTYPE.itemsize == 64 and HIT_DTYPE.itemsize == 32
+# rrt_ray_f32 (32 B) / rrt_hit_f32 (16 B): fp32 rays promoted exactly to f64 on the device, hits rounded to nearest
+RAY_F32_DTYPE = np.dtype([("o", "<f4", 3), ("t_max", "<f4"), ("d", "<f4", 3), ("reserved", "<u4")])
+HIT_F32_DTYPE = np.dtype([("prim_id", "<u4"), ("t", "<f4"), ("u", "<f4"), ("v", "<f4")])
+assert RAY_F32_DTYPE.itemsize == 32 and HIT_F32_DTYPE.itemsize == 16
 
 
 def _ptr(a):
@@ -34,6 +38,40 @@ def pack_rays(rays) -> np.ndarray:
     out = np.zeros((a.shape[0], 8), dtype=np.float64)
     out[:, : a.shape[1]] = a
     return out.view(RAY_DTYPE).reshape(-1)
+
+
+def pack_rays_f32(rays, out=None) -> np.ndarray:
+    """[n,7] float32 (o, d, t_max) -> rrt_ray_f32 records, into `out` when given (e.g. a `Context.pinned_empty` array).
+    f64 input is refused rather than rounded: what the fp32 entries answer for is the fp32 ray."""
+    if isinstance(rays, np.ndarray) and rays.dtype == RAY_F32_DTYPE:
+        if out is None:
+            return np.ascontiguousarray(rays)
+        out[:] = rays
+        return out
+    a = np.asarray(rays)
+    if a.dtype != np.float32:
+        raise TypeError(f"fp32 rays must be float32, got {a.dtype} (round them with .astype(np.float32) if that is meant)")
+    if a.ndim != 2 or a.shape[1] != 7:
+        raise ValueError("fp32 rays must be [n,7] (o, d, t_max)")
+    r = np.empty(a.shape[0], dtype=RAY_F32_DTYPE) if out is None else out
+    if r.shape != (a.shape[0],) or r.dtype != RAY_F32_DTYPE:
+        raise ValueError("out must be an rrt_ray_f32 array of the batch's length")
+    r["o"] = a[:, 0:3]
+    r["d"] = a[:, 3:6]
+    r["t_max"] = a[:, 6]
+    r["reserved"] = 0
+    return r
+
+
+def promote_rays_f32(rays) -> np.ndarray:
+    """The rrt_ray records an fp32 batch stands for (exact promotion, time = 0): the f64 call with these answers what
+    the fp32 call answers, before rounding."""
+    r = pack_rays_f32(rays)
+    out = np.zeros(r.shape[0], dtype=RAY_DTYPE)
+    out["o"] = r["o"]
+    out["d"] = r["d"]
+    out["t_max"] = r["t_max"]
+    return out
 
 
 class Context:
@@ -207,6 +245,23 @@ class GpuAggregate:
         capi.check(self.L.rrt_intersect_p(self.h, r.shape[0], _ptr(r), _ptr(occ)))
         return occ
 
+    # ---- the same over fp32 rays (rrt_ray_f32) and compact hits (rrt_hit_f32), HOST buffers ------------------
+    # For the link's full rate pass records in page-locked memory: rays packed with pack_rays_f32(a, out=...) and `out`,
+    # both from Context.pinned_empty (pageable buffers work, through a staging copy of the driver's).
+    def intersect_f32(self, rays, out=None) -> np.ndarray:
+        """`Scene::intersect` for an fp32 batch: [n,7] float32 or rrt_ray_f32 records in, HIT_F32_DTYPE records out."""
+        r = pack_rays_f32(rays)
+        hits = np.empty(r.shape[0], dtype=HIT_F32_DTYPE) if out is None else out
+        capi.check(self.L.rrt_intersect_f32(self.h, r.shape[0], _ptr(r), _ptr(hits)))
+        return hits
+
+    def intersect_p_f32(self, rays, out=None) -> np.ndarray:
+        """`Scene::intersect_p` for an fp32 batch: returns 0/1 bytes."""
+        r = pack_rays_f32(rays)
+        occ = np.empty(r.shape[0], dtype=np.uint8) if out is None else out
+        capi.check(self.L.rrt_intersect_p_f32(self.h, r.shape[0], _ptr(r), _ptr(occ)))
+        return occ
+
     # ---- same, DEVICE buffers (raw pointers; torch tensors' data_ptr()) ---------------------
     def intersect_device(self, n: int, d_rays: int, d_hits: int, stream: int = 0):
         capi.check(self.L.rrt_intersect_device(self.h, n, C.c_void_p(d_rays), C.c_void_p(d_hits), C.c_void_p(stream)))
@@ -214,6 +269,15 @@ class GpuAggregate:
     def intersect_p_device(self, n: int, d_rays: int, d_occluded: int, stream: int = 0):
         capi.check(self.L.rrt_intersect_p_device(self.h, n, C.c_void_p(d_rays), C.c_void_p(d_occluded),
                                                  C.c_void_p(stream)))
+
+    def intersect_f32_device(self, n: int, d_rays: int, d_hits: int, stream: int = 0):
+        """rrt_intersect_f32_device: n rrt_ray_f32 (32 B each) -> n rrt_hit_f32 (16 B each), 16-byte aligned device
+        buffers, asynchronous on `stream`."""
+        capi.check(self.L.rrt_intersect_f32_device(self.h, n, C.c_void_p(d_rays), C.c_void_p(d_hits), C.c_void_p(stream)))
+
+    def intersect_p_f32_device(self, n: int, d_rays: int, d_occluded: int, stream: int = 0):
+        capi.check(self.L.rrt_intersect_p_f32_device(self.h, n, C.c_void_p(d_rays), C.c_void_p(d_occluded),
+                                                     C.c_void_p(stream)))
 
 
 def lbvh_host_probe(bounds6: np.ndarray, max_prims_in_node: int = 4):
@@ -228,6 +292,18 @@ def lbvh_host_probe(bounds6: np.ndarray, max_prims_in_node: int = 4):
     cnt = C.c_uint32()
     capi.check(L.rrt_lbvh_host_probe(n, _ptr(b), max_prims_in_node, words.shape[0], C.byref(cnt), _ptr(words), _ptr(order), _ptr(info)))
     return words[: cnt.value], order, {"nodes": int(info[0]), "max_depth": int(info[1]), "leaves": int(info[2])}
+
+
+def rays_f32_host_probe(rays, hits):
+    """rrt_rays_f32_host_probe: the library's fp32 format conversions run on the host (CPU tests).
+    rays: RAY_F32_DTYPE records -> RAY_DTYPE as the walk sees them; hits: HIT_DTYPE -> HIT_F32_DTYPE."""
+    L = capi.lib()
+    r = np.ascontiguousarray(rays, dtype=RAY_F32_DTYPE)
+    h = np.ascontiguousarray(hits, dtype=HIT_DTYPE)
+    promoted = np.zeros(r.shape[0], dtype=RAY_DTYPE)
+    compact = np.zeros(h.shape[0], dtype=HIT_F32_DTYPE)
+    capi.check(L.rrt_rays_f32_host_probe(r.shape[0], _ptr(r), _ptr(promoted), h.shape[0], _ptr(h), _ptr(compact)))
+    return promoted, compact
 
 
 def soup_aggregate(ctx: Context, p, idx, max_prims_in_node: int = 4, build_flags: int = capi.RRT_BUILD_FAST) -> GpuAggregate:

@@ -77,6 +77,11 @@ def lib() -> C.CDLL:
         "rrt_intersect_p_device": (i32, [vp, u64, vp, vp, vp]),
         "rrt_intersect": (i32, [vp, u64, vp, vp]),
         "rrt_intersect_p": (i32, [vp, u64, vp, vp]),
+        "rrt_intersect_f32_device": (i32, [vp, u64, vp, vp, vp]),
+        "rrt_intersect_p_f32_device": (i32, [vp, u64, vp, vp, vp]),
+        "rrt_intersect_f32": (i32, [vp, u64, vp, vp]),
+        "rrt_intersect_p_f32": (i32, [vp, u64, vp, vp]),
+        "rrt_rays_f32_host_probe": (i32, [u64, vp, vp, u64, vp, vp]),
         "rrt_tri_screen_host_probe": (i32, [u64, vp, vp, vp, vp, vp]),
         "rrt_scene_update_instances": (i32, [vp, u32, u32, vp, vp]),
         "rrt_scene_export_tree": (i32, [vp, vp, u64, C.POINTER(u64)]),

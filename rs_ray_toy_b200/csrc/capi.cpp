@@ -8,6 +8,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <memory>
 #include <mutex>
 #include <new>
@@ -20,6 +21,8 @@
 #include "halton.cuh"
 #include "literal.hpp"
 #include "png_min.hpp"
+#include "rays_f32.cuh"
+#include "rays_f32.hpp"
 #include "render.hpp"
 #include "scene_json.hpp"
 #include "stratified.cuh"
@@ -83,6 +86,7 @@ struct Slot {
     cudaStream_t stream = nullptr;
     rrt_ray* d_rays = nullptr;
     void* d_out = nullptr;  // rrt_hit[kChunkRays] (also large enough for the any-hit bytes)
+    void* d_f32 = nullptr;  // fp32 calls only: the chunk's rrt_ray_f32, then its rrt_hit_f32 (the rays are dead by then)
 };
 
 }  // namespace
@@ -105,11 +109,18 @@ struct rrt_ctx {
         slots_ready = true;
         return RRT_OK;
     }
+    // added by the first fp32 call, so that callers of the f64 entries pay no memory for them
+    int ensure_f32_slots() {
+        for (auto& s : slots)
+            if (!s.d_f32) CAPI_CUDA(cudaMalloc(&s.d_f32, kChunkRays * sizeof(rrt_ray_f32)));
+        return RRT_OK;
+    }
     ~rrt_ctx() {
         cudaSetDevice(device);
         for (auto& s : slots) {
             if (s.d_rays) cudaFree(s.d_rays);
             if (s.d_out) cudaFree(s.d_out);
+            if (s.d_f32) cudaFree(s.d_f32);
             if (s.stream) cudaStreamDestroy(s.stream);
         }
     }
@@ -128,6 +139,33 @@ struct rrt_scene {
     uint32_t build_flags = 0;
     uint32_t max_prims_in_node = 4;
     std::atomic<int> live_renders{0};  // integrators made over this scene (they hold its aggregate and shading tables)
+
+    // rrt_intersect_f32_device / rrt_intersect_p_f32_device: the promoted rays and the f64 hits of a batch, one set per
+    // calling stream, grown to the largest batch seen there; past kMaxF32Scratch streams the first set is shared,
+    // ordered by its event (the policy of DeviceAggregate's workspaces).
+    struct F32Scratch {
+        rrt_ray* d_rays = nullptr;
+        rrt_hit* d_hits = nullptr;
+        uint64_t ray_capacity = 0, hit_capacity = 0;
+        cudaEvent_t last_use = nullptr;
+        bool used = false;
+        void* last_stream = nullptr;
+    };
+    static constexpr size_t kMaxF32Scratch = 8;
+    mutable std::mutex f32_mutex;
+    mutable std::map<void*, F32Scratch> f32_scratch;
+
+    ~rrt_scene() {
+        for (auto& kv : f32_scratch) {
+            F32Scratch& w = kv.second;
+            if (w.last_use) {
+                cudaEventSynchronize(w.last_use);
+                cudaEventDestroy(w.last_use);
+            }
+            if (w.d_rays) cudaFree(w.d_rays);
+            if (w.d_hits) cudaFree(w.d_hits);
+        }
+    }
 };
 
 struct rrt_render {
@@ -144,8 +182,11 @@ rrt::Transform xf_from(const double* m, const double* inv) {
     return t;
 }
 
-template <bool ANY>
-int host_batch(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, void* out) {
+// The host-buffer pipeline of both record formats.  F32: a chunk goes up as rrt_ray_f32 into the slot's staging
+// buffer and is promoted into the slot's rrt_ray buffer; its f64 hits are compacted into the staging buffer, whose
+// rays are dead by then, and go down from there.
+template <bool ANY, bool F32>
+int host_batch(const rrt_scene* scene, uint64_t n, const void* rays, void* out) {
     if (!scene || !scene->committed) return fail(RRT_ERR_INVALID, "scene is not committed");
     if (n == 0) return RRT_OK;
     if (!rays || !out) return fail(RRT_ERR_INVALID, "null ray / output buffer");
@@ -154,7 +195,12 @@ int host_batch(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, void* ou
     int rc = ctx->ensure_slots();
     if (rc != RRT_OK) return rc;
     CAPI_CUDA(cudaSetDevice(ctx->device));
-    const size_t out_elem = ANY ? sizeof(uint8_t) : sizeof(rrt_hit);
+    if (F32 && (rc = ctx->ensure_f32_slots()) != RRT_OK) return rc;
+    const size_t in_elem = F32 ? sizeof(rrt_ray_f32) : sizeof(rrt_ray);
+    const size_t out_elem = ANY ? sizeof(uint8_t) : (F32 ? sizeof(rrt_hit_f32) : sizeof(rrt_hit));
+    auto drain = [&] {  // copies of earlier chunks into the caller's buffer may still be in flight
+        for (auto& t : ctx->slots) cudaStreamSynchronize(t.stream);
+    };
     std::string err;
     uint64_t done = 0;
     int k = 0;
@@ -176,21 +222,42 @@ int host_batch(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, void* ou
         }
         mark(0, s.stream);
         // a slot is reused only after its previous D2H has drained (stream order)
-        CAPI_CUDA(cudaMemcpyAsync(s.d_rays, rays + done, cnt * sizeof(rrt_ray), cudaMemcpyHostToDevice, s.stream));
+        CAPI_CUDA(cudaMemcpyAsync(F32 ? s.d_f32 : s.d_rays, static_cast<const char*>(rays) + done * in_elem, cnt * in_elem,
+                                  cudaMemcpyHostToDevice, s.stream));
         mark(1, s.stream);
         int launched = 0;
+        if (F32) {
+            const int e = rrt::launch_promote_rays(cnt, static_cast<const rrt_ray_f32*>(s.d_f32), s.d_rays, s.stream);
+            if (e != cudaSuccess) {
+                drain();
+                return cuda_fail("promote_rays_kernel", (cudaError_t)e);
+            }
+            ++launched;
+        }
+        int traced = 0;
         if (ANY)
-            rc = scene->agg->any_hit(cnt, s.d_rays, static_cast<uint8_t*>(s.d_out), s.stream, &err, &launched);
+            rc = scene->agg->any_hit(cnt, s.d_rays, static_cast<uint8_t*>(s.d_out), s.stream, &err, &traced);
         else
-            rc = scene->agg->closest_hit(cnt, s.d_rays, static_cast<rrt_hit*>(s.d_out), s.stream, &err, &launched);
+            rc = scene->agg->closest_hit(cnt, s.d_rays, static_cast<rrt_hit*>(s.d_out), s.stream, &err, &traced);
         if (rc != RRT_OK) {
-            // copies of earlier chunks into the caller's buffer may still be in flight: drain them before returning
-            for (auto& t : ctx->slots) cudaStreamSynchronize(t.stream);
+            drain();
             return fail(rc, err);
+        }
+        launched += traced;
+        const void* d_result = s.d_out;
+        if (F32 && !ANY) {
+            const int e = rrt::launch_compact_hits(cnt, static_cast<const rrt_hit*>(s.d_out), static_cast<rrt_hit_f32*>(s.d_f32),
+                                                   s.stream);
+            if (e != cudaSuccess) {
+                drain();
+                return cuda_fail("compact_hits_kernel", (cudaError_t)e);
+            }
+            ++launched;
+            d_result = s.d_f32;
         }
         ctx->launches.fetch_add((uint64_t)launched, std::memory_order_relaxed);
         mark(2, s.stream);
-        CAPI_CUDA(cudaMemcpyAsync(static_cast<char*>(out) + done * out_elem, s.d_out, cnt * out_elem,
+        CAPI_CUDA(cudaMemcpyAsync(static_cast<char*>(out) + done * out_elem, d_result, cnt * out_elem,
                                   cudaMemcpyDeviceToHost, s.stream));
         mark(3, s.stream);
         done += cnt;
@@ -207,6 +274,63 @@ int host_batch(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, void* ou
         for (auto& m : marks)
             for (auto& e : m.e) cudaEventDestroy(e);
     }
+    return RRT_OK;
+}
+
+// rrt_intersect_f32_device / rrt_intersect_p_f32_device: promote into the stream's scratch, walk, compact into the
+// caller's buffer.  The scratch lock is held while the three passes are enqueued, so that a shared scratch's event
+// orders whole calls.
+template <bool ANY>
+int device_f32(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, void* d_out, void* stream, const char* name) {
+    if (!scene || !scene->committed) return fail(RRT_ERR_INVALID, std::string(name) + ": scene is not committed");
+    if (n == 0) return RRT_OK;
+    if (!d_rays || !d_out) return fail(RRT_ERR_INVALID, std::string(name) + ": null buffer");
+    if (n >= (1ull << 32)) return fail(RRT_ERR_INVALID, std::string(name) + ": batch too large for one call (2^32 rays)");
+    if ((reinterpret_cast<uintptr_t>(d_rays) | (ANY ? 0 : reinterpret_cast<uintptr_t>(d_out))) & 15u)
+        return fail(RRT_ERR_INVALID, std::string(name) + ": device buffers must be 16-byte aligned");
+    CAPI_CUDA(cudaSetDevice(scene->ctx->device));
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    std::lock_guard<std::mutex> lock(scene->f32_mutex);
+    auto& pool = scene->f32_scratch;
+    rrt_scene::F32Scratch& w =
+        (pool.count(stream) || pool.size() < rrt_scene::kMaxF32Scratch) ? pool[stream] : pool.begin()->second;
+    if (!w.last_use) CAPI_CUDA(cudaEventCreateWithFlags(&w.last_use, cudaEventDisableTiming));
+    if (n > w.ray_capacity || (!ANY && n > w.hit_capacity)) {
+        // the buffers are replaced: every call that used them is ordered before the last one (same stream, or the event)
+        if (w.used) CAPI_CUDA(cudaEventSynchronize(w.last_use));
+        if (n > w.ray_capacity) {
+            if (w.d_rays) cudaFree(w.d_rays);
+            w.d_rays = nullptr;
+            w.ray_capacity = 0;
+            CAPI_CUDA(cudaMalloc(&w.d_rays, n * sizeof(rrt_ray)));
+            w.ray_capacity = n;
+        }
+        if (!ANY && n > w.hit_capacity) {
+            if (w.d_hits) cudaFree(w.d_hits);
+            w.d_hits = nullptr;
+            w.hit_capacity = 0;
+            CAPI_CUDA(cudaMalloc(&w.d_hits, n * sizeof(rrt_hit)));
+            w.hit_capacity = n;
+        }
+    }
+    if (w.used && w.last_stream != stream) CAPI_CUDA(cudaStreamWaitEvent(s, w.last_use, 0));
+    int e = rrt::launch_promote_rays(n, d_rays, w.d_rays, stream);
+    if (e != cudaSuccess) return cuda_fail("promote_rays_kernel", (cudaError_t)e);
+    std::string err;
+    int launched = 0;
+    const int rc = ANY ? scene->agg->any_hit(n, w.d_rays, static_cast<uint8_t*>(d_out), stream, &err, &launched)
+                       : scene->agg->closest_hit(n, w.d_rays, w.d_hits, stream, &err, &launched);
+    if (rc != RRT_OK) return fail(rc, err);
+    launched += 1;
+    if (!ANY) {
+        e = rrt::launch_compact_hits(n, w.d_hits, static_cast<rrt_hit_f32*>(d_out), stream);
+        if (e != cudaSuccess) return cuda_fail("compact_hits_kernel", (cudaError_t)e);
+        launched += 1;
+    }
+    CAPI_CUDA(cudaEventRecord(w.last_use, s));
+    w.used = true;
+    w.last_stream = stream;
+    scene->ctx->launches.fetch_add((uint64_t)launched, std::memory_order_relaxed);
     return RRT_OK;
 }
 
@@ -991,10 +1115,32 @@ int rrt_render_hit_dump(rrt_render* render, int enable, double* out, uint64_t ca
 }
 
 int rrt_intersect(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, rrt_hit* hits) {
-    return host_batch<false>(scene, n, rays, hits);
+    return host_batch<false, false>(scene, n, rays, hits);
 }
 int rrt_intersect_p(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, uint8_t* occluded) {
-    return host_batch<true>(scene, n, rays, occluded);
+    return host_batch<true, false>(scene, n, rays, occluded);
+}
+int rrt_intersect_f32(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* rays, rrt_hit_f32* hits) {
+    return host_batch<false, true>(scene, n, rays, hits);
+}
+int rrt_intersect_p_f32(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* rays, uint8_t* occluded) {
+    return host_batch<true, true>(scene, n, rays, occluded);
+}
+int rrt_intersect_f32_device(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, rrt_hit_f32* d_hits,
+                             void* cuda_stream) {
+    return device_f32<false>(scene, n, d_rays, d_hits, cuda_stream, "rrt_intersect_f32_device");
+}
+int rrt_intersect_p_f32_device(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, uint8_t* d_occluded,
+                               void* cuda_stream) {
+    return device_f32<true>(scene, n, d_rays, d_occluded, cuda_stream, "rrt_intersect_p_f32_device");
+}
+int rrt_rays_f32_host_probe(uint64_t n_rays, const rrt_ray_f32* rays, rrt_ray* promoted, uint64_t n_hits, const rrt_hit* hits,
+                            rrt_hit_f32* compact) {
+    if ((n_rays && (!rays || !promoted)) || (n_hits && (!hits || !compact)))
+        return fail(RRT_ERR_INVALID, "rrt_rays_f32_host_probe: null argument");
+    for (uint64_t i = 0; i < n_rays; ++i) promoted[i] = rrt::promote_ray(rays[i]);
+    for (uint64_t i = 0; i < n_hits; ++i) compact[i] = rrt::compact_hit(hits[i]);
+    return RRT_OK;
 }
 
 int rrt_tri_screen_host_probe(uint64_t n, const double* o3, const double* d3, const double* best_t, const float* verts9,

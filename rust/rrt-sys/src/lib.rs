@@ -27,6 +27,12 @@ pub struct rrt_ray { pub o: [f64; 3], pub d: [f64; 3], pub t_max: f64, pub time:
 /// what BVHAccel::intersect hands back through `r.t_max` and `si`
 #[repr(C)] #[derive(Copy, Clone, Debug, Default)]
 pub struct rrt_hit { pub prim_id: u32, pub reserved: u32, pub t: f64, pub u: f64, pub v: f64 }
+/// fp32 ray for rrt_intersect_f32 and relatives: promoted exactly to `rrt_ray` (time 0) on the device
+#[repr(C)] #[derive(Copy, Clone, Debug, Default)]
+pub struct rrt_ray_f32 { pub o: [f32; 3], pub t_max: f32, pub d: [f32; 3], pub reserved: u32 }
+/// `rrt_hit` with t, u, v rounded to nearest fp32
+#[repr(C)] #[derive(Copy, Clone, Debug, Default)]
+pub struct rrt_hit_f32 { pub prim_id: u32, pub t: f32, pub u: f32, pub v: f32 }
 
 /// material/{matte,plastic,metal,mirror,glass,translucent,disney,debug_material}.rs with constant parameters
 /// (kind: 0 Matte .. 4 Glass, 5 Translucent, 6 Disney, 7 Debug)
@@ -88,6 +94,9 @@ const _: () = assert!(size_of::<rrt_material>() == 304);
 const _: () = assert!(size_of::<rrt_texture>() == 312);
 const _: () = assert!(size_of::<rrt_light>() == 624);
 const _: () = assert!(size_of::<rrt_render_desc>() == 256);
+// the fp32 records (tests/test_rays_f32.py checks these sizes against the C side)
+const _: () = assert!(size_of::<rrt_ray_f32>() == 32);
+const _: () = assert!(size_of::<rrt_hit_f32>() == 16);
 
 extern "C" {
     // ---- context ----
@@ -120,6 +129,11 @@ extern "C" {
     pub fn rrt_intersect_p_device(scene: *const rrt_scene, n: u64, d_rays: *const rrt_ray, d_occluded: *mut u8, cuda_stream: *mut c_void) -> c_int;
     pub fn rrt_intersect(scene: *const rrt_scene, n: u64, rays: *const rrt_ray, hits: *mut rrt_hit) -> c_int;
     pub fn rrt_intersect_p(scene: *const rrt_scene, n: u64, rays: *const rrt_ray, occluded: *mut u8) -> c_int;
+    // ---- the same over fp32 rays and compact hits ----
+    pub fn rrt_intersect_f32(scene: *const rrt_scene, n: u64, rays: *const rrt_ray_f32, hits: *mut rrt_hit_f32) -> c_int;
+    pub fn rrt_intersect_p_f32(scene: *const rrt_scene, n: u64, rays: *const rrt_ray_f32, occluded: *mut u8) -> c_int;
+    pub fn rrt_intersect_f32_device(scene: *const rrt_scene, n: u64, d_rays: *const rrt_ray_f32, d_hits: *mut rrt_hit_f32, cuda_stream: *mut c_void) -> c_int;
+    pub fn rrt_intersect_p_f32_device(scene: *const rrt_scene, n: u64, d_rays: *const rrt_ray_f32, d_occluded: *mut u8, cuda_stream: *mut c_void) -> c_int;
     // ---- shading tables ----
     pub fn rrt_scene_set_materials(scene: *mut rrt_scene, n: u32, materials: *const rrt_material) -> c_int;
     pub fn rrt_scene_set_lights(scene: *mut rrt_scene, n: u32, lights: *const rrt_light) -> c_int;
