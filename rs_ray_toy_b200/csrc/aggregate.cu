@@ -1173,7 +1173,26 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
         SahParams sp;
         sp.max_leaf = max_prims_in_node == 0 ? 4 : max_prims_in_node;
         if (const char* e = std::getenv("RRT_SAH_CI")) sp.cost_intersect = atof(e);
-        build_sah(AabbSpan(boxes, n), sp, &tree);
+        // spatial splits (DESIGN.md §3); RRT_SBVH_CAP=1 builds the object-split tree, one reference per primitive
+        if (const char* e = std::getenv("RRT_SBVH_ALPHA")) sp.split_alpha = atof(e);
+        if (const char* e = std::getenv("RRT_SBVH_CAP")) sp.split_cap = atof(e);
+        // spatial splits clip the triangles' world-space vertices; spheres stay whole references
+        RawBuf<uint8_t> is_tri(n);
+        bool all_tri = true;
+        for (size_t i = 0; i < n; ++i) {
+            is_tri[i] = scene.prims[i].kind == SHAPE_TRIANGLE ? 1 : 0;
+            all_tri = all_tri && is_tri[i];
+        }
+        SplitTriangles tris;
+        tris.verts = world.get()->v;  // (World is nine doubles: primitive i's vertices start at 9 i)
+        tris.is_tri = all_tri ? nullptr : is_tri.get();
+        build_sah(AabbSpan(boxes, n), tris, sp, &tree);
+        if (tree.max_depth + 2 > (uint32_t)kStack) {
+            // duplicated references can deepen a tree past the traversal stack; the object-split tree splits every
+            // node by count at worst, and is the one such a scene gets
+            tree = Bvh2();
+            build_sah(AabbSpan(boxes, n), sp, &tree);
+        }
     }
     if (tree.max_depth + 2 > (uint32_t)kStack) {
         if (on_device_ok) cudaFree(lb.d_nodes);
@@ -1186,8 +1205,11 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
     std::vector<Node64> nodes;
     nodes.reserve(tree.nodes.size() / 2 + 2);
     const bool wide = !all_fp32;
-    RawBuf<PrimRec48> rec48(wide ? 0 : n);  // every slot is written below: one record per primitive
-    RawBuf<PrimRec96> rec96(wide ? n : 0);
+    // one record per leaf reference (the device tree and the object-split host tree: one per primitive; spatial splits
+    // reference a triangle from every leaf that holds a part of it) — every slot is written below
+    const size_t n_refs = on_device_ok ? n : tree.order.size();
+    RawBuf<PrimRec48> rec48(wide ? 0 : n_refs);
+    RawBuf<PrimRec96> rec96(wide ? n_refs : 0);
     size_t n_rec = 0;  // host tree: records are appended leaf by leaf
     auto make_record = [&](uint32_t pi, size_t slot) {
         {
@@ -1352,7 +1374,7 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
     RRT_CUDA(cudaSetDevice(device));
     const size_t node_bytes = on_device_ok ? lb.node_bytes : (quantise ? nodes32.size() * sizeof(Node32) : nodes.size() * sizeof(Node64));
     const void* node_src = quantise ? (const void*)nodes32.data() : (const void*)nodes.data();
-    size_t prim_bytes = wide ? n * sizeof(PrimRec96) : n * sizeof(PrimRec48);
+    size_t prim_bytes = wide ? n_refs * sizeof(PrimRec96) : n_refs * sizeof(PrimRec48);
     if (on_device_ok) {
         d_nodes_ = lb.d_nodes;
     } else {
@@ -1418,7 +1440,7 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
     stats_.n_leaves = tree.n_leaves;
     stats_.max_depth = tree.max_depth;
     stats_.device_bytes = node_bytes + prim_bytes;
-    stats_.n_records = n;
+    stats_.n_records = n_refs;
     stats_.wide_records = wide;
     stats_.n_prims = n;
     stats_.build_usec =

@@ -44,7 +44,9 @@ struct NoInitAlloc : std::allocator<T> {
 
 struct Bvh2 {
     std::vector<Bvh2Node, NoInitAlloc<Bvh2Node>> nodes;
-    std::vector<uint32_t> order;  // primitive indices, leaf ranges are contiguous
+    // primitive indices, leaf ranges are contiguous; with spatial splits a primitive may appear in several leaves, so this
+    // holds the references (as many as nodes[root].n_prims), not one entry per primitive
+    std::vector<uint32_t> order;
     uint32_t root = 0;
     uint32_t max_depth = 0;
     uint32_t n_leaves = 0;
@@ -55,8 +57,24 @@ struct SahParams {
     double cost_traverse = 1.0;
     double cost_intersect = 2.0;
     int n_threads = 0;          // 0 = hardware_concurrency
+    // Spatial splits (SBVH, Stich et al. 2009), used only when the builder is given triangle vertices: a node tries one
+    // when its best object split's children overlap by more than split_alpha x the root's surface area, and the tree
+    // holds at most split_cap x n references.  (DESIGN.md §3: measured on configs 3 and 5.)
+    double split_alpha = 1e-5;
+    double split_cap = 1.3;
 };
 
+// World-space triangle vertices for spatial splits: primitive i's are verts[9 i .. 9 i + 8] (v0, v1, v2) when
+// is_tri is null or is_tri[i] != 0.  Other primitives (spheres) stay whole references.
+struct SplitTriangles {
+    const double* verts = nullptr;
+    const uint8_t* is_tri = nullptr;
+};
+
+// object splits only: one reference per primitive
 void build_sah(AabbSpan boxes, const SahParams& params, Bvh2* out);
+// object and spatial splits: triangles may be referenced from several leaves, each time with the box of the part of
+// the triangle inside that leaf
+void build_sah(AabbSpan boxes, const SplitTriangles& tris, const SahParams& params, Bvh2* out);
 
 }  // namespace rrt
