@@ -77,6 +77,20 @@ typedef struct rrt_hit_f32 {
     float v;
 } rrt_hit_f32;
 
+/* What BVHAccel::intersect leaves in `si` for the winning primitive (primitives.rs:56-57, interaction.rs:85-113), world
+ * space, f64: the fields Shape::intersect fills (triangle.rs with its shading geometry, sphere.rs:127-255), carried through
+ * a TransformedPrimitive's transform (primitives.rs:126-139, transform.rs:604-656).  A triangle's geometric dndu / dndv are
+ * zero; a sphere's are its Weingarten values, which `shading` copies.  On a miss `hit` is rrt_intersect's miss record and
+ * every other field is +0.0.  p_error is not carried: the reference always leaves it zero (interaction.rs:154); nor are
+ * time, the ray differentials or the primitive (prim_id names it).  336 bytes, 42 doubles.                             */
+typedef struct rrt_surface {
+    rrt_hit hit;                 /* byte for byte what rrt_intersect returns for this ray                 */
+    double p[3], wo[3], n[3];    /* BaseInteraction                                                       */
+    double uv[2];
+    double dpdu[3], dpdv[3], dndu[3], dndv[3];
+    double sh_n[3], sh_dpdu[3], sh_dpdv[3], sh_dndu[3], sh_dndv[3]; /* SurfaceInteraction::shading         */
+} rrt_surface;
+
 /* BVHSplitMethod (bvh.rs:111-114) plus the parity tier (SURVEY.md §8c).                         */
 typedef enum rrt_build_flags {
     RRT_BUILD_FAST = 0,    /* Tier F: own SAH tree, true closest hit, ties -> lowest prim id     */
@@ -181,6 +195,21 @@ int rrt_intersect_f32_device(const rrt_scene* scene, uint64_t n, const rrt_ray_f
                              void* cuda_stream);
 int rrt_intersect_p_f32_device(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, uint8_t* d_occluded,
                                void* cuda_stream);
+
+/* Scene::intersect with both of Primitive::intersect's outputs (primitives.rs:56-57): the hit and the SurfaceInteraction
+ * the reference fills for it, one rrt_surface per ray.  surfaces[i].hit equals rrt_intersect's record for ray i bit for
+ * bit, in both tiers and for every build flag.  Errors, limits and threading are those of rrt_intersect /
+ * rrt_intersect_device.  The first surface call on a scene uploads its shape tables (the mesh arrays, spheres and
+ * instance transforms; the literal tier's aggregate already holds them), kept until rrt_scene_destroy;
+ * rrt_scene_update_instances refreshes them.
+ * Device buffers, asynchronous on `cuda_stream`: the f64 hits of the batch live in scratch memory the scene keeps per
+ * calling stream, 32 bytes per ray, shared with the fp32 entries' scratch (same growth, eight streams, event order).
+ * Host buffers: the chunked pipeline of rrt_intersect, in chunks of at most a quarter of its chunk (256 Ki rays); the
+ * first surface call on a context adds an 84 MiB record buffer to each of its four slots (336 MiB of device memory,
+ * kept until rrt_destroy).                                                                                              */
+int rrt_intersect_surface_device(const rrt_scene* scene, uint64_t n, const rrt_ray* d_rays, rrt_surface* d_surfaces,
+                                 void* cuda_stream);
+int rrt_intersect_surface(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, rrt_surface* surfaces);
 
 /* ---- the render loop ------------------------------------------------------------------------
  * What deploy_render builds and runs (renderprocess.rs:92-105): make_scene + make_integrator,

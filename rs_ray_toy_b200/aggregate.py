@@ -22,6 +22,12 @@ assert RAY_DTYPE.itemsize == 64 and HIT_DTYPE.itemsize == 32
 RAY_F32_DTYPE = np.dtype([("o", "<f4", 3), ("t_max", "<f4"), ("d", "<f4", 3), ("reserved", "<u4")])
 HIT_F32_DTYPE = np.dtype([("prim_id", "<u4"), ("t", "<f4"), ("u", "<f4"), ("v", "<f4")])
 assert RAY_F32_DTYPE.itemsize == 32 and HIT_F32_DTYPE.itemsize == 16
+# rrt_surface (336 B): the hit and the SurfaceInteraction the reference fills for it, world space (interaction.rs:85-113)
+SURFACE_DTYPE = np.dtype([("hit", HIT_DTYPE), ("p", "<f8", 3), ("wo", "<f8", 3), ("n", "<f8", 3), ("uv", "<f8", 2),
+                          ("dpdu", "<f8", 3), ("dpdv", "<f8", 3), ("dndu", "<f8", 3), ("dndv", "<f8", 3),
+                          ("sh_n", "<f8", 3), ("sh_dpdu", "<f8", 3), ("sh_dpdv", "<f8", 3), ("sh_dndu", "<f8", 3),
+                          ("sh_dndv", "<f8", 3)])
+assert SURFACE_DTYPE.itemsize == 336
 
 
 def _ptr(a):
@@ -262,6 +268,16 @@ class GpuAggregate:
         capi.check(self.L.rrt_intersect_p_f32(self.h, r.shape[0], _ptr(r), _ptr(occ)))
         return occ
 
+    def intersect_surface(self, rays, out=None) -> np.ndarray:
+        """`Scene::intersect` with the SurfaceInteraction of each hit (primitives.rs:56-57): SURFACE_DTYPE records, whose
+        `hit` is what `intersect` returns.  For the link's full rate pass `out` from Context.pinned_empty."""
+        r = pack_rays(rays)
+        surfaces = np.empty(r.shape[0], dtype=SURFACE_DTYPE) if out is None else out
+        if surfaces.dtype != SURFACE_DTYPE or surfaces.shape != (r.shape[0],):
+            raise ValueError("out must be an rrt_surface array of the batch's length")
+        capi.check(self.L.rrt_intersect_surface(self.h, r.shape[0], _ptr(r), _ptr(surfaces)))
+        return surfaces
+
     # ---- same, DEVICE buffers (raw pointers; torch tensors' data_ptr()) ---------------------
     def intersect_device(self, n: int, d_rays: int, d_hits: int, stream: int = 0):
         capi.check(self.L.rrt_intersect_device(self.h, n, C.c_void_p(d_rays), C.c_void_p(d_hits), C.c_void_p(stream)))
@@ -269,6 +285,11 @@ class GpuAggregate:
     def intersect_p_device(self, n: int, d_rays: int, d_occluded: int, stream: int = 0):
         capi.check(self.L.rrt_intersect_p_device(self.h, n, C.c_void_p(d_rays), C.c_void_p(d_occluded),
                                                  C.c_void_p(stream)))
+
+    def intersect_surface_device(self, n: int, d_rays: int, d_surfaces: int, stream: int = 0):
+        """rrt_intersect_surface_device: n rrt_ray (64 B each) -> n rrt_surface (336 B each), asynchronous on `stream`."""
+        capi.check(self.L.rrt_intersect_surface_device(self.h, n, C.c_void_p(d_rays), C.c_void_p(d_surfaces),
+                                                       C.c_void_p(stream)))
 
     def intersect_f32_device(self, n: int, d_rays: int, d_hits: int, stream: int = 0):
         """rrt_intersect_f32_device: n rrt_ray_f32 (32 B each) -> n rrt_hit_f32 (16 B each), 16-byte aligned device

@@ -26,6 +26,7 @@
 #include "render.hpp"
 #include "scene_json.hpp"
 #include "stratified.cuh"
+#include "surface.hpp"
 #include "tri_screen.h"
 #include "rrt_test.h"
 
@@ -59,18 +60,22 @@ uint64_t chunk_rays() {
     return v;
 }
 #define kChunkRays (chunk_rays())
+// rays per pipeline slot of the surface calls: a quarter of the chunk, so that the slots' 336-byte records take 84 MiB
+// each instead of 336 MiB.  Their chunks are bound by the records' D2H, not by the walk, so a smaller chunk costs nothing
+// that the four-slot pipeline does not hide.
+uint64_t surface_chunk_rays() { return kChunkRays / 4; }
 // The pipeline's fill (first H2D, nothing to trace yet) and drain (last kernel + D2H, nothing left to upload) are each one
 // chunk long, so the chunks at both ends of a batch are small and double towards the middle: 128 Ki, 128 Ki, 256 Ki, 512 Ki,
 // 1 Mi ... 1 Mi, 512 Ki, 256 Ki, 128 Ki.  Measured on a 16 Mi-ray batch: 701 -> 726 Mrays/s (profiles/r2_e2e_taper.txt); the
 // link's own floor for 1 GiB up + 0.5 GiB down at once is 20.5 ms = 819 Mrays/s (profiles/r2_pcie_probe.txt), and the
 // uploads run at 49.5 GB/s while hits stream down (55.5 GB/s alone): 21.7 ms + the last chunk's walk (0.5 ms: a batch of
 // any size takes that long) is what is left (profiles/r2_e2e_trace.txt).  RRT_HOST_TAPER=0: off.
-uint64_t tapered_chunk(uint64_t done, uint64_t n) {
+uint64_t tapered_chunk(uint64_t done, uint64_t n, uint64_t full) {
     static const bool taper = [] {
         const char* e = std::getenv("RRT_HOST_TAPER");
         return !(e && e[0] == '0');
     }();
-    const uint64_t full = kChunkRays, left = n - done;
+    const uint64_t left = n - done;
     uint64_t c = full;
     if (taper) {
         const uint64_t floor_c = full >> 3 ? full >> 3 : 1;
@@ -87,6 +92,7 @@ struct Slot {
     rrt_ray* d_rays = nullptr;
     void* d_out = nullptr;  // rrt_hit[kChunkRays] (also large enough for the any-hit bytes)
     void* d_f32 = nullptr;  // fp32 calls only: the chunk's rrt_ray_f32, then its rrt_hit_f32 (the rays are dead by then)
+    void* d_surf = nullptr; // surface calls only: the chunk's rrt_surface records
 };
 
 }  // namespace
@@ -115,12 +121,19 @@ struct rrt_ctx {
             if (!s.d_f32) CAPI_CUDA(cudaMalloc(&s.d_f32, kChunkRays * sizeof(rrt_ray_f32)));
         return RRT_OK;
     }
+    // likewise added by the first surface call
+    int ensure_surface_slots() {
+        for (auto& s : slots)
+            if (!s.d_surf) CAPI_CUDA(cudaMalloc(&s.d_surf, surface_chunk_rays() * sizeof(rrt_surface)));
+        return RRT_OK;
+    }
     ~rrt_ctx() {
         cudaSetDevice(device);
         for (auto& s : slots) {
             if (s.d_rays) cudaFree(s.d_rays);
             if (s.d_out) cudaFree(s.d_out);
             if (s.d_f32) cudaFree(s.d_f32);
+            if (s.d_surf) cudaFree(s.d_surf);
             if (s.stream) cudaStreamDestroy(s.stream);
         }
     }
@@ -140,10 +153,11 @@ struct rrt_scene {
     uint32_t max_prims_in_node = 4;
     std::atomic<int> live_renders{0};  // integrators made over this scene (they hold its aggregate and shading tables)
 
-    // rrt_intersect_f32_device / rrt_intersect_p_f32_device: the promoted rays and the f64 hits of a batch, one set per
-    // calling stream, grown to the largest batch seen there; past kMaxF32Scratch streams the first set is shared,
-    // ordered by its event (the policy of DeviceAggregate's workspaces).
-    struct F32Scratch {
+    // The device entries that run more than the walk (rrt_intersect_f32_device, rrt_intersect_p_f32_device,
+    // rrt_intersect_surface_device): the promoted rays and / or the f64 hits of a batch, one set per calling stream, grown
+    // to the largest batch seen there; past kMaxScratch streams the first set is shared, ordered by its event (the policy
+    // of DeviceAggregate's workspaces).  acquire_scratch / release_scratch below.
+    struct StreamScratch {
         rrt_ray* d_rays = nullptr;
         rrt_hit* d_hits = nullptr;
         uint64_t ray_capacity = 0, hit_capacity = 0;
@@ -151,13 +165,18 @@ struct rrt_scene {
         bool used = false;
         void* last_stream = nullptr;
     };
-    static constexpr size_t kMaxF32Scratch = 8;
-    mutable std::mutex f32_mutex;
-    mutable std::map<void*, F32Scratch> f32_scratch;
+    static constexpr size_t kMaxScratch = 8;
+    mutable std::mutex scratch_mutex;
+    mutable std::map<void*, StreamScratch> scratch;
+
+    // the surface pass's shape tables (Tier F), uploaded by the first surface call; the literal tier reads its
+    // aggregate's own
+    mutable std::mutex surface_mutex;
+    mutable rrt::SurfaceTables* surface_tables = nullptr;
 
     ~rrt_scene() {
-        for (auto& kv : f32_scratch) {
-            F32Scratch& w = kv.second;
+        for (auto& kv : scratch) {
+            StreamScratch& w = kv.second;
             if (w.last_use) {
                 cudaEventSynchronize(w.last_use);
                 cudaEventDestroy(w.last_use);
@@ -165,6 +184,7 @@ struct rrt_scene {
             if (w.d_rays) cudaFree(w.d_rays);
             if (w.d_hits) cudaFree(w.d_hits);
         }
+        rrt::surface_tables_destroy(surface_tables);
     }
 };
 
@@ -182,10 +202,29 @@ rrt::Transform xf_from(const double* m, const double* inv) {
     return t;
 }
 
-// The host-buffer pipeline of both record formats.  F32: a chunk goes up as rrt_ray_f32 into the slot's staging
+// The surface pass's tables: the literal tier's own, or the scene's, uploaded on first use (Tier F).
+int surface_tables(const rrt_scene* scene, const rrt::ShadeScene** tables, bool* literal) {
+    if (scene->build_flags == RRT_BUILD_LITERAL) {
+        *tables = &static_cast<const rrt::LiteralAggregate*>(scene->agg.get())->geometry_tables();
+        *literal = true;
+        return RRT_OK;
+    }
+    std::lock_guard<std::mutex> lock(scene->surface_mutex);
+    if (!scene->surface_tables) {
+        std::string err;
+        const int rc = rrt::surface_tables_create(scene->host, &scene->surface_tables, &err);
+        if (rc != RRT_OK) return fail(rc, err);
+    }
+    *tables = rrt::surface_tables_view(scene->surface_tables);
+    *literal = false;
+    return RRT_OK;
+}
+
+// The host-buffer pipeline of every record format.  F32: a chunk goes up as rrt_ray_f32 into the slot's staging
 // buffer and is promoted into the slot's rrt_ray buffer; its f64 hits are compacted into the staging buffer, whose
-// rays are dead by then, and go down from there.
-template <bool ANY, bool F32>
+// rays are dead by then, and go down from there.  SURF: the surface pass turns the chunk's rays and f64 hits into
+// rrt_surface records in the slot's record buffer, in chunks of surface_chunk_rays().
+template <bool ANY, bool F32, bool SURF = false>
 int host_batch(const rrt_scene* scene, uint64_t n, const void* rays, void* out) {
     if (!scene || !scene->committed) return fail(RRT_ERR_INVALID, "scene is not committed");
     if (n == 0) return RRT_OK;
@@ -196,8 +235,13 @@ int host_batch(const rrt_scene* scene, uint64_t n, const void* rays, void* out) 
     if (rc != RRT_OK) return rc;
     CAPI_CUDA(cudaSetDevice(ctx->device));
     if (F32 && (rc = ctx->ensure_f32_slots()) != RRT_OK) return rc;
+    const rrt::ShadeScene* tables = nullptr;
+    bool literal = false;
+    if (SURF && ((rc = ctx->ensure_surface_slots()) != RRT_OK || (rc = surface_tables(scene, &tables, &literal)) != RRT_OK))
+        return rc;
+    const uint64_t full_chunk = SURF ? surface_chunk_rays() : kChunkRays;
     const size_t in_elem = F32 ? sizeof(rrt_ray_f32) : sizeof(rrt_ray);
-    const size_t out_elem = ANY ? sizeof(uint8_t) : (F32 ? sizeof(rrt_hit_f32) : sizeof(rrt_hit));
+    const size_t out_elem = ANY ? sizeof(uint8_t) : (F32 ? sizeof(rrt_hit_f32) : (SURF ? sizeof(rrt_surface) : sizeof(rrt_hit)));
     auto drain = [&] {  // copies of earlier chunks into the caller's buffer may still be in flight
         for (auto& t : ctx->slots) cudaStreamSynchronize(t.stream);
     };
@@ -215,7 +259,7 @@ int host_batch(const rrt_scene* scene, uint64_t n, const void* rays, void* out) 
     };
     while (done < n) {
         Slot& s = ctx->slots[k % kSlots];
-        const uint64_t cnt = tapered_chunk(done, n);
+        const uint64_t cnt = tapered_chunk(done, n, full_chunk);
         if (tracing) {
             marks.push_back(Marks{});
             marks.back().cnt = cnt;
@@ -255,6 +299,16 @@ int host_batch(const rrt_scene* scene, uint64_t n, const void* rays, void* out) 
             ++launched;
             d_result = s.d_f32;
         }
+        if (SURF) {
+            const int e = rrt::launch_surfaces(*tables, literal, cnt, s.d_rays, static_cast<const rrt_hit*>(s.d_out),
+                                               static_cast<rrt_surface*>(s.d_surf), s.stream);
+            if (e != cudaSuccess) {
+                drain();
+                return cuda_fail("surface_kernel", (cudaError_t)e);
+            }
+            ++launched;
+            d_result = s.d_surf;
+        }
         ctx->launches.fetch_add((uint64_t)launched, std::memory_order_relaxed);
         mark(2, s.stream);
         CAPI_CUDA(cudaMemcpyAsync(static_cast<char*>(out) + done * out_elem, d_result, cnt * out_elem,
@@ -277,9 +331,45 @@ int host_batch(const rrt_scene* scene, uint64_t n, const void* rays, void* out) 
     return RRT_OK;
 }
 
+// The calling stream's scratch (rrt_scene::StreamScratch), with room for `n_rays` promoted rays and `n_hits` f64 hits,
+// and `stream` ordered after the last call that used it.  Called with scene->scratch_mutex held, which the caller keeps
+// while it enqueues its passes and until release_scratch, so that a shared scratch's event orders whole calls.
+int acquire_scratch(const rrt_scene* scene, void* stream, uint64_t n_rays, uint64_t n_hits, rrt_scene::StreamScratch** out) {
+    auto& pool = scene->scratch;
+    rrt_scene::StreamScratch& w =
+        (pool.count(stream) || pool.size() < rrt_scene::kMaxScratch) ? pool[stream] : pool.begin()->second;
+    if (!w.last_use) CAPI_CUDA(cudaEventCreateWithFlags(&w.last_use, cudaEventDisableTiming));
+    if (n_rays > w.ray_capacity || n_hits > w.hit_capacity) {
+        // the buffers are replaced: every call that used them is ordered before the last one (same stream, or the event)
+        if (w.used) CAPI_CUDA(cudaEventSynchronize(w.last_use));
+        if (n_rays > w.ray_capacity) {
+            if (w.d_rays) cudaFree(w.d_rays);
+            w.d_rays = nullptr;
+            w.ray_capacity = 0;
+            CAPI_CUDA(cudaMalloc(&w.d_rays, n_rays * sizeof(rrt_ray)));
+            w.ray_capacity = n_rays;
+        }
+        if (n_hits > w.hit_capacity) {
+            if (w.d_hits) cudaFree(w.d_hits);
+            w.d_hits = nullptr;
+            w.hit_capacity = 0;
+            CAPI_CUDA(cudaMalloc(&w.d_hits, n_hits * sizeof(rrt_hit)));
+            w.hit_capacity = n_hits;
+        }
+    }
+    if (w.used && w.last_stream != stream) CAPI_CUDA(cudaStreamWaitEvent(static_cast<cudaStream_t>(stream), w.last_use, 0));
+    *out = &w;
+    return RRT_OK;
+}
+int release_scratch(rrt_scene::StreamScratch* w, void* stream) {
+    CAPI_CUDA(cudaEventRecord(w->last_use, static_cast<cudaStream_t>(stream)));
+    w->used = true;
+    w->last_stream = stream;
+    return RRT_OK;
+}
+
 // rrt_intersect_f32_device / rrt_intersect_p_f32_device: promote into the stream's scratch, walk, compact into the
-// caller's buffer.  The scratch lock is held while the three passes are enqueued, so that a shared scratch's event
-// orders whole calls.
+// caller's buffer.
 template <bool ANY>
 int device_f32(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, void* d_out, void* stream, const char* name) {
     if (!scene || !scene->committed) return fail(RRT_ERR_INVALID, std::string(name) + ": scene is not committed");
@@ -289,47 +379,51 @@ int device_f32(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, vo
     if ((reinterpret_cast<uintptr_t>(d_rays) | (ANY ? 0 : reinterpret_cast<uintptr_t>(d_out))) & 15u)
         return fail(RRT_ERR_INVALID, std::string(name) + ": device buffers must be 16-byte aligned");
     CAPI_CUDA(cudaSetDevice(scene->ctx->device));
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    std::lock_guard<std::mutex> lock(scene->f32_mutex);
-    auto& pool = scene->f32_scratch;
-    rrt_scene::F32Scratch& w =
-        (pool.count(stream) || pool.size() < rrt_scene::kMaxF32Scratch) ? pool[stream] : pool.begin()->second;
-    if (!w.last_use) CAPI_CUDA(cudaEventCreateWithFlags(&w.last_use, cudaEventDisableTiming));
-    if (n > w.ray_capacity || (!ANY && n > w.hit_capacity)) {
-        // the buffers are replaced: every call that used them is ordered before the last one (same stream, or the event)
-        if (w.used) CAPI_CUDA(cudaEventSynchronize(w.last_use));
-        if (n > w.ray_capacity) {
-            if (w.d_rays) cudaFree(w.d_rays);
-            w.d_rays = nullptr;
-            w.ray_capacity = 0;
-            CAPI_CUDA(cudaMalloc(&w.d_rays, n * sizeof(rrt_ray)));
-            w.ray_capacity = n;
-        }
-        if (!ANY && n > w.hit_capacity) {
-            if (w.d_hits) cudaFree(w.d_hits);
-            w.d_hits = nullptr;
-            w.hit_capacity = 0;
-            CAPI_CUDA(cudaMalloc(&w.d_hits, n * sizeof(rrt_hit)));
-            w.hit_capacity = n;
-        }
-    }
-    if (w.used && w.last_stream != stream) CAPI_CUDA(cudaStreamWaitEvent(s, w.last_use, 0));
-    int e = rrt::launch_promote_rays(n, d_rays, w.d_rays, stream);
+    std::lock_guard<std::mutex> lock(scene->scratch_mutex);
+    rrt_scene::StreamScratch* w = nullptr;
+    int rc = acquire_scratch(scene, stream, n, ANY ? 0 : n, &w);
+    if (rc != RRT_OK) return rc;
+    int e = rrt::launch_promote_rays(n, d_rays, w->d_rays, stream);
     if (e != cudaSuccess) return cuda_fail("promote_rays_kernel", (cudaError_t)e);
     std::string err;
     int launched = 0;
-    const int rc = ANY ? scene->agg->any_hit(n, w.d_rays, static_cast<uint8_t*>(d_out), stream, &err, &launched)
-                       : scene->agg->closest_hit(n, w.d_rays, w.d_hits, stream, &err, &launched);
+    rc = ANY ? scene->agg->any_hit(n, w->d_rays, static_cast<uint8_t*>(d_out), stream, &err, &launched)
+             : scene->agg->closest_hit(n, w->d_rays, w->d_hits, stream, &err, &launched);
     if (rc != RRT_OK) return fail(rc, err);
     launched += 1;
     if (!ANY) {
-        e = rrt::launch_compact_hits(n, w.d_hits, static_cast<rrt_hit_f32*>(d_out), stream);
+        e = rrt::launch_compact_hits(n, w->d_hits, static_cast<rrt_hit_f32*>(d_out), stream);
         if (e != cudaSuccess) return cuda_fail("compact_hits_kernel", (cudaError_t)e);
         launched += 1;
     }
-    CAPI_CUDA(cudaEventRecord(w.last_use, s));
-    w.used = true;
-    w.last_stream = stream;
+    if ((rc = release_scratch(w, stream)) != RRT_OK) return rc;
+    scene->ctx->launches.fetch_add((uint64_t)launched, std::memory_order_relaxed);
+    return RRT_OK;
+}
+
+// rrt_intersect_surface_device: walk into the stream's scratch hits, then the surface pass into the caller's records.
+int device_surface(const rrt_scene* scene, uint64_t n, const rrt_ray* d_rays, rrt_surface* d_out, void* stream) {
+    const char* name = "rrt_intersect_surface_device";
+    if (!scene || !scene->committed) return fail(RRT_ERR_INVALID, std::string(name) + ": scene is not committed");
+    if (n == 0) return RRT_OK;
+    if (!d_rays || !d_out) return fail(RRT_ERR_INVALID, std::string(name) + ": null buffer");
+    if (n >= (1ull << 32)) return fail(RRT_ERR_INVALID, std::string(name) + ": batch too large for one call (2^32 rays)");
+    CAPI_CUDA(cudaSetDevice(scene->ctx->device));
+    const rrt::ShadeScene* tables = nullptr;
+    bool literal = false;
+    int rc = surface_tables(scene, &tables, &literal);
+    if (rc != RRT_OK) return rc;
+    std::lock_guard<std::mutex> lock(scene->scratch_mutex);
+    rrt_scene::StreamScratch* w = nullptr;
+    if ((rc = acquire_scratch(scene, stream, 0, n, &w)) != RRT_OK) return rc;
+    std::string err;
+    int launched = 0;
+    rc = scene->agg->closest_hit(n, d_rays, w->d_hits, stream, &err, &launched);
+    if (rc != RRT_OK) return fail(rc, err);
+    const int e = rrt::launch_surfaces(*tables, literal, n, d_rays, w->d_hits, d_out, stream);
+    if (e != cudaSuccess) return cuda_fail("surface_kernel", (cudaError_t)e);
+    launched += 1;
+    if ((rc = release_scratch(w, stream)) != RRT_OK) return rc;
     scene->ctx->launches.fetch_add((uint64_t)launched, std::memory_order_relaxed);
     return RRT_OK;
 }
@@ -531,6 +625,10 @@ int rrt_scene_update_instances(rrt_scene* scene, uint32_t first_instance, uint32
         if (rc != RRT_OK) return fail(rc, err);
         scene->agg = std::move(fresh);
         scene->build_flags = RRT_BUILD_DEVICE_LBVH;
+        // the surface pass's tables hold the old transforms: the next surface call uploads them anew
+        std::lock_guard<std::mutex> lock(scene->surface_mutex);
+        rrt::surface_tables_destroy(scene->surface_tables);
+        scene->surface_tables = nullptr;
     } catch (const std::exception& e) {
         return fail(RRT_ERR_INVALID, e.what());
     }
@@ -1133,6 +1231,13 @@ int rrt_intersect_f32_device(const rrt_scene* scene, uint64_t n, const rrt_ray_f
 int rrt_intersect_p_f32_device(const rrt_scene* scene, uint64_t n, const rrt_ray_f32* d_rays, uint8_t* d_occluded,
                                void* cuda_stream) {
     return device_f32<true>(scene, n, d_rays, d_occluded, cuda_stream, "rrt_intersect_p_f32_device");
+}
+int rrt_intersect_surface(const rrt_scene* scene, uint64_t n, const rrt_ray* rays, rrt_surface* surfaces) {
+    return host_batch<false, false, true>(scene, n, rays, surfaces);
+}
+int rrt_intersect_surface_device(const rrt_scene* scene, uint64_t n, const rrt_ray* d_rays, rrt_surface* d_surfaces,
+                                 void* cuda_stream) {
+    return device_surface(scene, n, d_rays, d_surfaces, cuda_stream);
 }
 int rrt_rays_f32_host_probe(uint64_t n_rays, const rrt_ray_f32* rays, rrt_ray* promoted, uint64_t n_hits, const rrt_hit* hits,
                             rrt_hit_f32* compact) {

@@ -294,6 +294,8 @@ int launch_literal(const LitView& v, uint64_t n, const rrt_ray* rays, rrt_hit* h
 }
 }  // namespace
 
+const ShadeScene& LiteralAggregate::geometry_tables() const { return impl_->view.sc; }
+
 int LiteralAggregate::closest_hit(uint64_t n, const rrt_ray* r, rrt_hit* h, void* s, std::string* err, int* l) const {
     return launch_literal<false>(impl_->view, n, r, h, nullptr, s, nullptr, err, l);
 }

@@ -11,6 +11,8 @@
 
 namespace rrt {
 
+struct ShadeScene;
+
 class LiteralAggregate : public RayTracer {
   public:
     LiteralAggregate() = default;
@@ -26,6 +28,8 @@ class LiteralAggregate : public RayTracer {
                          void* stream, std::string* err, int* launches = nullptr) const override;
     const AggregateStats& stats() const override { return stats_; }
     bool literal() const override { return true; }
+    // the geometry tables its shape tests read (scene_tables.cuh), which the surface pass reads too
+    const ShadeScene& geometry_tables() const;
     void root_bounds(double out6[6]) const {
         for (int k = 0; k < 6; ++k) out6[k] = root_bounds_[k];
     }

@@ -164,9 +164,19 @@ static __device__ __noinline__ void sphere_bump_partials(const SphereInfo& sp, V
     xf_surface_bump_partials(sp.o2w, sp.w2o, bp);
 }
 
+// The geometric dndu / dndv of a SurfaceInteraction (interaction.rs:85-113): only the intersect API's surface records carry
+// them.  Zero for triangles (Triangle::intersect hands SurfaceInteraction::new zero vectors); a sphere's are the Weingarten
+// values that sphere_bump_partials computes for its shading frame (SurfaceInteraction::new copies them into `shading`).
+struct GeomNormalPartials {
+    V3 dndu, dndv;
+};
+
 // Rebuilds the surface frame of hit (prim_id, t, u, v) for the world ray (o, d).
+// FULL = false (the renderer): uv / dpdu / dpdv only for scenes with textures, the shading partials only when `bp` is given.
+// FULL = true (rrt_intersect_surface): every field of the SurfaceInteraction; `bp` and `gp` must be given.
+template <bool FULL = false>
 __device__ __forceinline__ void make_surface_body(const ShadeScene& sc, uint32_t prim_id, double t, double bu, double bv, V3 o, V3 d,
-                                                  Surface* out, BumpPartials* bp) {
+                                                  Surface* out, BumpPartials* bp, GeomNormalPartials* gp = nullptr) {
     const PrimInfo pi = sc.prims[prim_id];
     V3 lo = o, ld = d;
     if (pi.instance >= 0) {  // TransformedPrimitive::intersect (primitives.rs:126-139), Q6 fixed: d keeps its length
@@ -177,7 +187,7 @@ __device__ __forceinline__ void make_surface_body(const ShadeScene& sc, uint32_t
     }
     Surface s;
     s.material = pi.material;
-    const bool textured = sc.n_textures != 0;
+    const bool textured = FULL || sc.n_textures != 0;
     if ((pi.kind & kPrimKindMask) == 0) {
         const V3 p0 = ld3(sc.mesh_p, pi.gv[0]), p1 = ld3(sc.mesh_p, pi.gv[1]), p2 = ld3(sc.mesh_p, pi.gv[2]);
         MeshInfo mi = {};  // read only for meshes that carry uv or normals
@@ -225,6 +235,7 @@ __device__ __forceinline__ void make_surface_body(const ShadeScene& sc, uint32_t
             bp->shdpdv = dpdv;
             bp->shdndu = bp->shdndv = v3(0, 0, 0);
         }
+        if constexpr (FULL) gp->dndu = gp->dndv = v3(0, 0, 0);
         if (mi.has_n && mi.has_ni) {
             const uint32_t* ni = sc.mesh_ni + mi.ni_off + 3ull * pi.tri;
             const double* nb = sc.mesh_n + 3 * mi.n_off;
@@ -285,6 +296,10 @@ __device__ __forceinline__ void make_surface_body(const ShadeScene& sc, uint32_t
         const V3 dpdu = v3(-sp.phi_max * p.y, sp.phi_max * p.x, 0.0);
         const V3 dpdv = v3(p.z * cos_phi, p.z * sin_phi, -sp.radius * sin(theta)) * (sp.theta_max - sp.theta_min);
         if (bp) sphere_bump_partials(sp, p, dpdu, dpdv, cos_phi, sin_phi, bp);  // out of line: bump-mapped scenes only
+        if constexpr (FULL) {
+            gp->dndu = bp->shdndu;
+            gp->dndv = bp->shdndv;
+        }
         s.p = p;
         s.wo = -od;
         s.n = normalize(cross(dpdu, dpdv));
@@ -304,6 +319,10 @@ __device__ __forceinline__ void make_surface_body(const ShadeScene& sc, uint32_t
             xf_surface(x.m, x.inv, &s);  // primitives.rs:135-137
             if (textured) xf_surface_partials(x.m, &s);
             if (bp) xf_surface_bump_partials(x.m, x.inv, bp);
+            if constexpr (FULL) {
+                gp->dndu = xf_normal_inv(x.inv, gp->dndu);
+                gp->dndv = xf_normal_inv(x.inv, gp->dndv);
+            }
         }
     }
     *out = s;

@@ -33,6 +33,16 @@ pub struct rrt_ray_f32 { pub o: [f32; 3], pub t_max: f32, pub d: [f32; 3], pub r
 /// `rrt_hit` with t, u, v rounded to nearest fp32
 #[repr(C)] #[derive(Copy, Clone, Debug, Default)]
 pub struct rrt_hit_f32 { pub prim_id: u32, pub t: f32, pub u: f32, pub v: f32 }
+/// the hit and the SurfaceInteraction BVHAccel::intersect leaves in `si` for it (interaction.rs:85-113), world space;
+/// 336 bytes (tests/test_surface.py checks the layout against the C side)
+#[repr(C)] #[derive(Copy, Clone, Debug, Default)]
+pub struct rrt_surface {
+    pub hit: rrt_hit,
+    pub p: [f64; 3], pub wo: [f64; 3], pub n: [f64; 3],
+    pub uv: [f64; 2],
+    pub dpdu: [f64; 3], pub dpdv: [f64; 3], pub dndu: [f64; 3], pub dndv: [f64; 3],
+    pub sh_n: [f64; 3], pub sh_dpdu: [f64; 3], pub sh_dpdv: [f64; 3], pub sh_dndu: [f64; 3], pub sh_dndv: [f64; 3],
+}
 
 /// material/{matte,plastic,metal,mirror,glass,translucent,disney,debug_material}.rs with constant parameters
 /// (kind: 0 Matte .. 4 Glass, 5 Translucent, 6 Disney, 7 Debug)
@@ -134,6 +144,9 @@ extern "C" {
     pub fn rrt_intersect_p_f32(scene: *const rrt_scene, n: u64, rays: *const rrt_ray_f32, occluded: *mut u8) -> c_int;
     pub fn rrt_intersect_f32_device(scene: *const rrt_scene, n: u64, d_rays: *const rrt_ray_f32, d_hits: *mut rrt_hit_f32, cuda_stream: *mut c_void) -> c_int;
     pub fn rrt_intersect_p_f32_device(scene: *const rrt_scene, n: u64, d_rays: *const rrt_ray_f32, d_occluded: *mut u8, cuda_stream: *mut c_void) -> c_int;
+    // ---- Scene::intersect with the SurfaceInteraction of each hit ----
+    pub fn rrt_intersect_surface(scene: *const rrt_scene, n: u64, rays: *const rrt_ray, surfaces: *mut rrt_surface) -> c_int;
+    pub fn rrt_intersect_surface_device(scene: *const rrt_scene, n: u64, d_rays: *const rrt_ray, d_surfaces: *mut rrt_surface, cuda_stream: *mut c_void) -> c_int;
     // ---- shading tables ----
     pub fn rrt_scene_set_materials(scene: *mut rrt_scene, n: u32, materials: *const rrt_material) -> c_int;
     pub fn rrt_scene_set_lights(scene: *mut rrt_scene, n: u32, lights: *const rrt_light) -> c_int;
