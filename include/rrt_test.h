@@ -2,7 +2,7 @@
  *
  * These run pieces of the PRODUCT's own code on the host so that the CPU test-suite (`pytest -m "not gpu"`) can
  * check them without a device: the device LBVH builder's per-element code, the literal tier's HLBVH, the texture
- * evaluator, the Halton tables, compute_differentials, the scene.json loader, the fp32 triangle screen.  They are
+ * evaluator, the Halton tables, compute_differentials, the scene.json loader.  They are
  * checkers, not a CPU path: none of them traces a ray or renders a sample.  A Rust `rrt-sys` crate binds
  * include/rrt.h only; nothing here belongs in it.                                                                  */
 #ifndef RRT_TEST_H
@@ -54,13 +54,6 @@ int rrt_scene_json_probe(const char* path, const char* overrides_json, uint64_t 
  * the first max_materials materials and their RRT_MATERIAL_SLOTS texture indices each (may be NULL).          */
 int rrt_scene_json_texture_probe(const char* path, const char* overrides_json, uint32_t* n_textures, rrt_texture* textures,
                                  uint32_t max_materials, uint32_t* n_materials, rrt_material* materials, int32_t* slots);
-
-/* Host-only probe of the closest-hit kernel's fp32 triangle screen (csrc/tri_screen.h, the code trace_kernel runs
- * before the f64 Moller-Trumbore test): for each of n cases — ray origin o[3], direction d[3], best_t, and the
- * nine fp32 vertex coordinates of a PrimRec48 triangle — out[i] = 1 when the screen says "surely rejected", 0 when
- * it abstains.  The CPU tests check that every 1 is a candidate the f64 test turns down as well.                */
-int rrt_tri_screen_host_probe(uint64_t n, const double* o3, const double* d3, const double* best_t, const float* verts9,
-                              uint8_t* out);
 
 /* Host-only probe of the device StratifiedSampler (csrc/stratified.cuh, the code the kernels run): for one pixel the
  * 1D tables out1d[ndims][xs * ys], the 2D tables out2d[ndims][xs * ys][2] as PixelSampler::start_pixel leaves them, and

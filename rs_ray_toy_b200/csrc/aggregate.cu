@@ -20,6 +20,7 @@
 #include <atomic>
 #include <cstring>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "aggregate.hpp"
@@ -27,7 +28,6 @@
 #include "bvh_pack_plan.hpp"
 #include "device_layout.h"
 #include "sphere_core.cuh"
-#include "tri_screen.h"
 
 namespace rrt {
 
@@ -143,24 +143,9 @@ __device__ __forceinline__ bool slab(const RayF& r, float lox, float hix, float 
     return tmin <= tmax;
 }
 
-// Node32 variant: the ray's direction signs pick the near / far plane of every axis when the plane is decoded
-// (the PRMT selector), so no min / max pair per axis is needed.  w* hold lo | hi << 16 (device_layout.h).
-#ifndef RRT_SIGN_SELECT
-#define RRT_SIGN_SELECT 0  // measured slower: three more live registers -> spills at 64, fewer CTAs at 72 (profiles/r1_sweep13)
-#endif
-__device__ __forceinline__ bool slab_q(const RayF& r, uint32_t wx, uint32_t wy, uint32_t wz, uint32_t selx, uint32_t sely,
-                                       uint32_t selz, float tcull, float* tnear) {
-    const float nx = fmaf(__uint_as_float(__byte_perm(wx, 0x3Fu, selx)), r.idx, -r.oidx);
-    const float ny = fmaf(__uint_as_float(__byte_perm(wy, 0x3Fu, sely)), r.idy, -r.oidy);
-    const float nz = fmaf(__uint_as_float(__byte_perm(wz, 0x3Fu, selz)), r.idz, -r.oidz);
-    const float fx = fmaf(__uint_as_float(__byte_perm(wx, 0x3Fu, selx ^ 0x0220u)), r.idx, -r.oidx);
-    const float fy = fmaf(__uint_as_float(__byte_perm(wy, 0x3Fu, sely ^ 0x0220u)), r.idy, -r.oidy);
-    const float fz = fmaf(__uint_as_float(__byte_perm(wz, 0x3Fu, selz ^ 0x0220u)), r.idz, -r.oidz);
-    const float tmin = fmaxf(fmaxf(nx, ny), fmaxf(nz, 0.0f));
-    const float tmax = fminf(fminf(fx, fy), fminf(fz, tcull));
-    *tnear = tmin;
-    return tmin <= tmax;
-}
+// Node32 planes: a word holds lo | hi << 16 (device_layout.h); these decode the lo / hi plane
+__device__ __forceinline__ float qlo(uint32_t w) { return __uint_as_float(__byte_perm(w, 0x3Fu, 0x4105)); }
+__device__ __forceinline__ float qhi(uint32_t w) { return __uint_as_float(__byte_perm(w, 0x3Fu, 0x4325)); }
 
 template <bool WIDE>
 __device__ __forceinline__ void load_prim(const void* prims, uint32_t idx, D3* a, D3* b, D3* c, uint32_t* prim_id,
@@ -334,41 +319,26 @@ constexpr int32_t kNoLeaf = 0;         // leaf references are negative, so 0 mea
 #ifndef RRT_NODE32
 #define RRT_NODE32 1  // 0: never quantise, 1: per scene (quantise when the grid is fine enough), 2: always
 #endif
-#ifndef RRT_STALE_SKIP
-#define RRT_STALE_SKIP 0
-#endif
 #ifndef RRT_STATS
 #define RRT_STATS 0
 #endif
 #ifndef RRT_WALK_MIN
 #define RRT_WALK_MIN 12
 #endif
-#ifndef RRT_PREFETCH_FAR
-#define RRT_PREFETCH_FAR 0  // 1: prefetch.global.L2, 2: prefetch.global.L1 of the pushed child
-#endif
 #ifndef RRT_LEAF_MIN
 #define RRT_LEAF_MIN 8
-#endif
-#ifndef RRT_LEAF_TRIPS
-#define RRT_LEAF_TRIPS 0  // 0: the leaf phase empties every queue; k: at most k leaves per lane and phase
 #endif
 #ifndef RRT_LEAFQ
 #define RRT_LEAFQ 3  // postponed leaves per lane (measured: with one, 10 of 32 lanes stand at their second leaf)
 #endif
+static_assert(RRT_LEAFQ >= 2, "the leaf queue holds the head leaf and at least one more");
 #ifndef RRT_MINBLOCKS
 #define RRT_MINBLOCKS 7  // Node64 kernels: 72 registers
 #endif
 #ifndef RRT_MINBLOCKS_Q
 #define RRT_MINBLOCKS_Q 8  // Node32 kernels: 64 registers (measured best, profiles/r1_sweep8.txt)
 #endif
-#ifndef RRT_STAGE_TOP
-#define RRT_STAGE_TOP 0  // K > 0: the K topmost interior nodes (breadth-first) are copied to shared memory by every CTA and
-                         // read from there — north_star's "shared-memory staging of top-level nodes".  Measured and not
-                         // adopted (profiles/r2_sweep_stage_top.txt): those nodes are the hottest lines of L1 already.
-#endif
-constexpr int kStageTop = RRT_STAGE_TOP;
 constexpr int kRefill = RRT_REFILL;
-constexpr int kScreenRows = RRT_PRETEST ? 9 : 0;  // ScreenRay rows behind the traversal stack (tri_screen.h)
 
 
 // GEN: the scene holds spheres that need the object-space test (PRIM_SPHERE_GENERAL); every other scene runs the
@@ -379,7 +349,7 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
                                                         const uint32_t* __restrict__ perm,
                                                         const uint32_t* __restrict__ use_perm,
                                                         unsigned long long* __restrict__ cursor,
-                                                        const uint32_t* __restrict__ n_dev, int stack_levels) {
+                                                        const uint32_t* __restrict__ n_dev, int /*stack_levels*/) {
     const unsigned FULL = 0xffffffffu;
     if (n_dev) n = *n_dev;  // wavefront queues: the batch size lives on the device
     const unsigned lane = threadIdx.x & 31u;
@@ -389,42 +359,17 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
     // Traversal stack: entirely in shared memory, laid out [level][thread] so that 32 lanes at 32
     // different depths still hit 32 different banks (one wavefront per push / pop).  Level 0 holds
     // the "stack empty" marker, so a pop never needs an underflow test.  The launch sizes it from
-    // the tree depth (stack_levels * kBlock * 4 bytes of dynamic shared memory).
+    // the tree depth (trace_smem_bytes).
     extern __shared__ int32_t sstack[];
     int32_t* const my_stack = sstack + threadIdx.x;
-#if RRT_STALE_SKIP
-    // closest hit only: every pushed subtree remembers its entry distance, so that a pop can drop
-    // subtrees that a hit found meanwhile has put out of reach without fetching their node
-    float* const my_tstack = reinterpret_cast<float*>(sstack + stack_levels * kBlock) + threadIdx.x;
-#define RRT_POP()                                                      \
-    do {                                                               \
-        --sp;                                                          \
-        node = my_stack[sp * kBlock];                                  \
-    } while (!ANY && my_tstack[sp * kBlock] > tcull)
-#else
 #define RRT_POP()                     \
     do {                              \
         --sp;                         \
         node = my_stack[sp * kBlock]; \
     } while (0)
-#endif
-    // the fp32 screen's per-ray constants (ScreenRay) live behind the stack, [row][thread] as well: nine floats that
-    // are written once per ray and read once per screened record — registers are what this kernel is short of
-    float* const my_screen = reinterpret_cast<float*>(sstack + stack_levels * kBlock * (RRT_STALE_SKIP ? 2 : 1)) + threadIdx.x;
-#if RRT_STAGE_TOP
-    // the K topmost nodes (indices 0 .. K-1 after the host's breadth-first relabelling), one copy per CTA
-    uint4* const s_top = reinterpret_cast<uint4*>(sstack + (stack_levels * (RRT_STALE_SKIP ? 2 : 1) + kScreenRows) * kBlock);
-    if (QUANT) {
-        const uint4* src = static_cast<const uint4*>(A.nodes);
-        const int n_stage = A.n_staged;
-        for (int k = threadIdx.x; k < 2 * n_stage; k += kBlock) s_top[k] = __ldg(src + k);
-        __syncthreads();
-    }
-#endif
     int sp = 1;
     int32_t node = kDone;     // >= 0 interior index, < 0 leaf reference, kDone = nothing left
     int32_t leaf = kNoLeaf;   // parked leaf reference (head of the queue)
-#if RRT_LEAFQ > 1
     int32_t lq[RRT_LEAFQ - 1];  // further parked leaves: the walk goes on past RRT_LEAFQ untested leaves
 #pragma unroll
     for (int k = 0; k < RRT_LEAFQ - 1; ++k) lq[k] = kNoLeaf;
@@ -443,13 +388,11 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
             }                                              \
         }                                                  \
     } while (0)
-#endif
     bool have_ray = false;
     bool exhausted = false;   // the global queue is empty (warp-uniform)
     uint64_t ray_index = 0;
     D3 o = {0, 0, 0}, d = {0, 0, 0};
     RayF rf = {0, 0, 0, 0, 0, 0};
-    uint32_t selx = 0x4105u, sely = 0x4105u, selz = 0x4105u;  // Node32: PRMT selectors of the near planes
     double best_t = 0.0;
     float t_shift = 0.0f, tcull = 0.0f;
     uint32_t best_id = RRT_NO_HIT, best_rec = 0;
@@ -500,30 +443,12 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
                     have_ray = true;
                     sp = 1;
                     my_stack[0] = kDone;
-#if RRT_STALE_SKIP
-                    my_tstack[0] = -1.0f;  // the marker is never stale
-#endif
                     leaf = kNoLeaf;
-#if RRT_LEAFQ > 1
 #pragma unroll
                     for (int k = 0; k < RRT_LEAFQ - 1; ++k) lq[k] = kNoLeaf;
-#endif
-                    if (!WIDE && RRT_PRETEST) {
-                        const ScreenRay R = make_screen_ray(o.x, o.y, o.z, d.x, d.y, d.z);
-                        my_screen[0 * kBlock] = R.ox; my_screen[1 * kBlock] = R.oy; my_screen[2 * kBlock] = R.oz;
-                        my_screen[3 * kBlock] = R.dx; my_screen[4 * kBlock] = R.dy; my_screen[5 * kBlock] = R.dz;
-                        my_screen[6 * kBlock] = R.mo;
-                        my_screen[7 * kBlock] = R.md;
-                        my_screen[8 * kBlock] = R.kmd;
-                    }
                     const bool live = prepare_ray(A, o, d, best_t, &t_shift, &rf) && !(best_t < 0.0);
                     node = live ? A.root : kDone;
                     tcull = __double2float_ru(best_t - (double)t_shift);
-                    if (QUANT && RRT_SIGN_SELECT) {  // a negative direction meets the upper plane first
-                        selx = rf.idx < 0.0f ? 0x4325u : 0x4105u;
-                        sely = rf.idy < 0.0f ? 0x4325u : 0x4105u;
-                        selz = rf.idz < 0.0f ? 0x4325u : 0x4105u;
-                    }
                 }
             }
         }
@@ -551,31 +476,13 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
                 if (QUANT) {
                     // one 256-bit load: 12 quantised planes + two child references; a plane becomes the float
                     // 1 + q / 32768 with one byte permute (device_layout.h)
-#if RRT_STAGE_TOP
-                    F8 v;
-                    if (node < A.n_staged) {
-                        const uint4 lo = s_top[2 * node], hi = s_top[2 * node + 1];
-                        v = F8{__uint_as_float(lo.x), __uint_as_float(lo.y), __uint_as_float(lo.z), __uint_as_float(lo.w),
-                               __uint_as_float(hi.x), __uint_as_float(hi.y), __uint_as_float(hi.z), __uint_as_float(hi.w)};
-                    } else {
-                        v = ldg256(reinterpret_cast<const char*>(A.nodes) + (size_t)node * sizeof(Node32));
-                    }
-#else
                     const F8 v = ldg256(reinterpret_cast<const char*>(A.nodes) + (size_t)node * sizeof(Node32));
-#endif
                     const uint32_t w0 = __float_as_uint(v.a), w1 = __float_as_uint(v.b), w2 = __float_as_uint(v.c);
                     const uint32_t w3 = __float_as_uint(v.d), w4 = __float_as_uint(v.e), w5 = __float_as_uint(v.f);
                     ch_x = __float_as_int(v.g);
                     ch_y = __float_as_int(v.h);
-#define RRT_QLO(w) __uint_as_float(__byte_perm((w), 0x3Fu, 0x4105))
-#define RRT_QHI(w) __uint_as_float(__byte_perm((w), 0x3Fu, 0x4325))
-#if RRT_SIGN_SELECT
-                    h0 = slab_q(rf, w0, w1, w2, selx, sely, selz, tcull, &tn0);
-                    h1 = slab_q(rf, w3, w4, w5, selx, sely, selz, tcull, &tn1);
-#else
-                    h0 = slab(rf, RRT_QLO(w0), RRT_QHI(w0), RRT_QLO(w1), RRT_QHI(w1), RRT_QLO(w2), RRT_QHI(w2), tcull, &tn0);
-                    h1 = slab(rf, RRT_QLO(w3), RRT_QHI(w3), RRT_QLO(w4), RRT_QHI(w4), RRT_QLO(w5), RRT_QHI(w5), tcull, &tn1);
-#endif
+                    h0 = slab(rf, qlo(w0), qhi(w0), qlo(w1), qhi(w1), qlo(w2), qhi(w2), tcull, &tn0);
+                    h1 = slab(rf, qlo(w3), qhi(w3), qlo(w4), qhi(w4), qlo(w5), qhi(w5), tcull, &tn1);
                 } else {
                     const char* np = reinterpret_cast<const char*>(nodes + node);
                     const F8 lo = ldg256(np);        // c0 x/y slabs, c1 x/y slabs
@@ -590,38 +497,15 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
                 const bool both = h0 && h1;
                 const bool swap = !ANY && (tn1 < tn0);
                 const int32_t near_c = swap ? ch_y : ch_x, far_c = swap ? ch_x : ch_y;
-                if (both) {
-                    my_stack[sp * kBlock] = far_c;
-#if RRT_PREFETCH_FAR
-                    // the far child is popped later: start moving its node towards L1 / L2 now
-                    if (far_c >= 0) {
-                        const char* fp = reinterpret_cast<const char*>(A.nodes) + (size_t)far_c * (QUANT ? sizeof(Node32) : sizeof(Node64));
-#if RRT_PREFETCH_FAR == 1
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(fp));
-#else
-                        asm volatile("prefetch.global.L1 [%0];" ::"l"(fp));
-#endif
-                    }
-#endif
-#if RRT_STALE_SKIP
-                    if (!ANY) my_tstack[sp * kBlock] = swap ? tn0 : tn1;
-#endif
-                }
+                if (both) my_stack[sp * kBlock] = far_c;
                 sp += both ? 1 : 0;
                 node = both ? near_c : (h0 ? ch_x : ch_y);
                 if (!(h0 || h1)) RRT_POP();
             }
-#if RRT_LEAFQ > 1
             if (node < 0 && lq[RRT_LEAFQ - 2] == kNoLeaf) {  // park the leaf, keep walking
                 RRT_PARK();
                 RRT_POP();
             }
-#else
-            if (node < 0 && leaf == kNoLeaf) {  // park the first leaf, keep walking
-                leaf = node;
-                RRT_POP();
-            }
-#endif
           }
             // leave when no lane is still looking for its first leaf
             if (!__any_sync(FULL, leaf == kNoLeaf && node != kDone)) break;
@@ -633,10 +517,7 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
         }
 
         // ---- leaf phase ----
-#if RRT_LEAF_TRIPS > 0
-#pragma unroll 1
-        for (int trip = 0; trip < RRT_LEAF_TRIPS && __any_sync(FULL, leaf != kNoLeaf); ++trip) {
-#elif RRT_LEAF_MIN > 0
+#if RRT_LEAF_MIN > 0
         // a leaf trip is worth its ~150 f64 instructions only with enough lanes in it: below RRT_LEAF_MIN the
         // remaining leaves stay queued while the others walk on — unless nobody is left to walk
         for (;;) {
@@ -653,27 +534,8 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
             if (leaf != kNoLeaf) {
                 const uint32_t ref = ~(uint32_t)leaf;
                 const uint32_t first = ref >> 3, cnt = (ref & 7u) + 1u;
-                // phase A (fp32-exact records only): screen every record of the leaf in fp32; what is left over
-                // goes to the f64 tests of phase B.  Spheres are never screened.
+                // every record of the leaf through the deciding arithmetic: f64, reference operation order
                 uint32_t cand = (1u << cnt) - 1u;
-                if (!WIDE && RRT_PRETEST) {
-                    ScreenRay R;
-                    R.ox = my_screen[0 * kBlock]; R.oy = my_screen[1 * kBlock]; R.oz = my_screen[2 * kBlock];
-                    R.dx = my_screen[3 * kBlock]; R.dy = my_screen[4 * kBlock]; R.dz = my_screen[5 * kBlock];
-                    R.mo = my_screen[6 * kBlock];
-                    R.md = my_screen[7 * kBlock];
-                    R.kmd = my_screen[8 * kBlock];
-                    R.bt = __double2float_ru(best_t);  // closest so far, or the shadow ray's t_max
-                    cand = 0u;
-                    for (uint32_t k = 0; k < cnt; ++k) {
-                        const float4* p = reinterpret_cast<const float4*>(static_cast<const PrimRec48*>(A.prims) + first + k);
-                        const float4 r0 = __ldg(p), r1 = __ldg(p + 1), r2 = __ldg(p + 2);
-                        const bool out = __float_as_uint(r2.z) == PRIM_TRIANGLE &&
-                                         tri_surely_missed(R, V4f{r0.x, r0.y, r0.z, r0.w}, V4f{r1.x, r1.y, r1.z, r1.w}, V4f{r2.x, r2.y, r2.z, r2.w});
-                        cand |= out ? 0u : (1u << k);
-                    }
-                }
-                // phase B: the deciding arithmetic, f64, reference operation order
                 while (cand != 0u) {
                     const uint32_t k = (uint32_t)__ffs((int)cand) - 1u;
                     cand &= cand - 1u;
@@ -703,7 +565,6 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
                         }
                     }
                 }
-#if RRT_LEAFQ > 1
                 leaf = lq[0];
 #pragma unroll
                 for (int k = 0; k < RRT_LEAFQ - 2; ++k) lq[k] = lq[k + 1];
@@ -717,15 +578,6 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
                     RRT_PARK();
                     RRT_POP();
                 }
-#else
-                leaf = kNoLeaf;
-                if (ANY && found) {
-                    node = kDone;
-                } else if (node < 0) {  // the walk had already reached another leaf
-                    leaf = node;
-                    RRT_POP();
-                }
-#endif
             }
         }
     }
@@ -740,6 +592,8 @@ __global__ void __launch_bounds__(kBlock, QUANT ? RRT_MINBLOCKS_Q : RRT_MINBLOCK
         atomicAdd(cursor + 8, st_lact);
     }
 #endif
+#undef RRT_POP
+#undef RRT_PARK
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -903,6 +757,24 @@ __global__ void __launch_bounds__(256) sort_scatter_kernel(uint64_t n, const uin
         perm[bins[k] + block_sums[k / kScanBlock] + rank[i]] = (uint32_t)i;
     }
 }
+
+// ---- trace_kernel launch facts: which instantiation, how much dynamic shared memory ----
+using TraceKernel = decltype(&trace_kernel<false, false, false, false>);
+
+// table[wide | any << 1 | quant << 2 | gen << 3]
+template <int... V>
+TraceKernel trace_kernel_table(int v, std::integer_sequence<int, V...>) {
+    static const TraceKernel table[] = {trace_kernel<(V & 2) != 0, (V & 1) != 0, (V & 4) != 0, (V & 8) != 0>...};
+    return table[v];
+}
+// The instantiation that serves one launch: any hit or closest hit, PrimRec96 records, Node32 nodes, general spheres.
+TraceKernel trace_kernel_for(bool any, bool wide, bool quant, bool gen) {
+    return trace_kernel_table((wide ? 1 : 0) | (any ? 2 : 0) | (quant ? 4 : 0) | (gen ? 8 : 0),
+                              std::make_integer_sequence<int, 16>{});
+}
+
+// The traversal stack, stack_levels entries per thread, is all of trace_kernel's dynamic shared memory.
+size_t trace_smem_bytes(int stack_levels) { return (size_t)stack_levels * kBlock * sizeof(int32_t); }
 
 inline float round_down(double v) {
     float f = (float)v;
@@ -1313,32 +1185,6 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
         }
     }
 
-    // ---- RRT_STAGE_TOP experiment: the K topmost interior nodes first, in breadth-first order ----
-    int n_staged = 0;
-    if (kStageTop > 0 && quantise && !on_device_ok && nodes.size() > (size_t)kStageTop) {
-        std::vector<uint32_t> top;
-        top.push_back(0);
-        for (size_t h = 0; h < top.size() && top.size() < (size_t)kStageTop; ++h) {
-            const Node64& nd = nodes[top[h]];
-            if (nd.child0 >= 0 && top.size() < (size_t)kStageTop) top.push_back((uint32_t)nd.child0);
-            if (nd.child1 >= 0 && top.size() < (size_t)kStageTop) top.push_back((uint32_t)nd.child1);
-        }
-        std::vector<int32_t> new_index(nodes.size(), -1);
-        for (size_t k = 0; k < top.size(); ++k) new_index[top[k]] = (int32_t)k;
-        int32_t next = (int32_t)top.size();
-        for (size_t i = 0; i < nodes.size(); ++i)
-            if (new_index[i] < 0) new_index[i] = next++;
-        std::vector<Node64> moved(nodes.size());
-        for (size_t i = 0; i < nodes.size(); ++i) {
-            Node64 nd = nodes[i];
-            if (nd.child0 >= 0) nd.child0 = new_index[nd.child0];
-            if (nd.child1 >= 0) nd.child1 = new_index[nd.child1];
-            moved[new_index[i]] = nd;
-        }
-        nodes.swap(moved);
-        n_staged = (int)top.size();
-    }
-    view_.n_staged = n_staged;
     // ---- quantise the host tree: Node64 (fp32 planes) -> Node32 (15-bit planes on the grid) ----
     std::vector<Node32> nodes32;
     if (quantise && !on_device_ok) {
@@ -1400,22 +1246,6 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
     }
     view_.gspheres = d_gspheres_;
     lap("upload");
-    // Optional (RRT_L2_PERSIST=1): a persisting L2 access-policy window over the nodes, against the ray / hit
-    // streams that pass through L2 (1.5 GB per 16 Mi-ray batch).  Measured: no gain (1443 vs 1466 Mrays/s,
-    // profiles/r1_sweep14) — the streams already use evict-first loads / stores — so it is off by default.
-    l2_window_bytes_ = 0;
-    {
-        const char* e = std::getenv("RRT_L2_PERSIST");
-        int max_persist = 0, max_window = 0;
-        cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, device);
-        cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, device);
-        if (e && atoi(e) != 0 && max_persist > 0 && max_window > 0) {
-            const size_t want = std::min<size_t>(node_bytes, (size_t)max_window);
-            cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, std::min<size_t>((size_t)max_persist, want));
-            l2_window_bytes_ = want;
-            l2_hit_ratio_ = (float)std::min(1.0, (double)std::min<size_t>((size_t)max_persist, want) / (double)want);
-        }
-    }
     view_.inst_w2p = static_cast<const double*>(d_inst_);
     view_.has_spheres = has_spheres ? 1 : 0;
     view_.nodes = d_nodes_;
@@ -1454,20 +1284,14 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
     return RRT_OK;
 }
 
-// the only shared memory is the traversal stack (one entry per tree level + the marker, [+ the screen's rows]);
+// the only shared memory is the traversal stack (one entry per tree level + the marker, trace_smem_bytes);
 // everything else of the 256 KB stays L1
 void DeviceAggregate::configure_kernels(bool quantise) {
-    const size_t smem = ((size_t)stack_levels_ * (RRT_STALE_SKIP ? 2 : 1) + kScreenRows) * kBlock * sizeof(int32_t) + (size_t)kStageTop * sizeof(Node32);
+    const size_t smem = trace_smem_bytes(stack_levels_);
     int carve = (int)(((quantise ? RRT_MINBLOCKS_Q : RRT_MINBLOCKS) * smem * 100 + 227 * 1024 - 1) / (227 * 1024)) + 2;
     if (carve > 100) carve = 100;
-    for (auto fn : {(const void*)trace_kernel<false, false, false, false>, (const void*)trace_kernel<false, true, false, false>,
-                    (const void*)trace_kernel<true, false, false, false>, (const void*)trace_kernel<true, true, false, false>,
-                    (const void*)trace_kernel<false, false, true, false>, (const void*)trace_kernel<false, true, true, false>,
-                    (const void*)trace_kernel<true, false, true, false>, (const void*)trace_kernel<true, true, true, false>,
-                    (const void*)trace_kernel<false, false, false, true>, (const void*)trace_kernel<false, true, false, true>,
-                    (const void*)trace_kernel<true, false, false, true>, (const void*)trace_kernel<true, true, false, true>,
-                    (const void*)trace_kernel<false, false, true, true>, (const void*)trace_kernel<false, true, true, true>,
-                    (const void*)trace_kernel<true, false, true, true>, (const void*)trace_kernel<true, true, true, true>}) {
+    for (int v = 0; v < 16; ++v) {
+        const void* fn = (const void*)trace_kernel_for(v & 1, v & 2, v & 4, v & 8);
         cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
     }
@@ -1481,6 +1305,7 @@ struct BlobHeader {
     int32_t stack_levels, sort_rays;
     uint64_t node_bytes, prim_bytes, inst_bytes, gsphere_bytes;
 };
+static_assert(sizeof(BlobHeader) == 280, "BlobHeader layout changed: bump the blob version");
 constexpr uint64_t kBlobMagic = 0x3130454552545252ull;  // "RRTREE01"
 }  // namespace
 
@@ -1634,28 +1459,14 @@ int DeviceAggregate::trace(uint64_t n, const rrt_ray* d_rays, rrt_hit* d_hits, u
                                                n_dev);
         count += 4;
     }
-    auto kernel = view_.gspheres != nullptr
-                      ? (view_.quantised ? (view_.wide ? trace_kernel<ANY, true, true, true> : trace_kernel<ANY, false, true, true>)
-                                         : (view_.wide ? trace_kernel<ANY, true, false, true> : trace_kernel<ANY, false, false, true>))
-                      : (view_.quantised ? (view_.wide ? trace_kernel<ANY, true, true, false> : trace_kernel<ANY, false, true, false>)
-                                         : (view_.wide ? trace_kernel<ANY, true, false, false> : trace_kernel<ANY, false, false, false>));
-    const size_t smem = ((size_t)stack_levels_ * (RRT_STALE_SKIP ? 2 : 1) + kScreenRows) * kBlock * sizeof(int32_t) + (size_t)kStageTop * sizeof(Node32);
+    const TraceKernel kernel = trace_kernel_for(ANY, view_.wide != 0, view_.quantised != 0, view_.gspheres != nullptr);
+    const size_t smem = trace_smem_bytes(stack_levels_);
     int per_sm = 0;
     RRT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kBlock, smem));
     if (per_sm < 1) per_sm = 1;
     uint64_t blocks = (uint64_t)w.n_sms * (uint64_t)per_sm;
     const uint64_t needed = (n + kBlock - 1) / kBlock;
     if (blocks > needed) blocks = needed;
-    if (l2_window_bytes_ && w.window_stream != s) {
-        cudaStreamAttrValue attr{};
-        attr.accessPolicyWindow.base_ptr = d_nodes_;
-        attr.accessPolicyWindow.num_bytes = l2_window_bytes_;
-        attr.accessPolicyWindow.hitRatio = l2_hit_ratio_;
-        attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        cudaStreamSetAttribute(s, cudaStreamAttributeAccessPolicyWindow, &attr);
-        w.window_stream = s;
-    }
     kernel<<<(unsigned)blocks, kBlock, smem, s>>>(view_, n, d_rays, d_hits, d_occ, sorting ? w.d_perm : nullptr,
                                                sorting ? small + 3 : nullptr,
                                                reinterpret_cast<unsigned long long*>(small), n_dev, stack_levels_);

@@ -35,8 +35,10 @@ struct AggView {
     int32_t wide;        // 1 => PrimRec96
     int32_t has_spheres;
     int32_t sort_mode;   // ray-queue key: 0 cell, 1 cell|octant, 2 octant|cell
-    int32_t n_staged;    // RRT_STAGE_TOP builds: nodes [0, n_staged) are the topmost ones in breadth-first order
+    int32_t reserved;    // always 0
 };
+// a kernel parameter, and copied whole into the header of an exported tree: its layout is part of the blob format
+static_assert(sizeof(AggView) == 152, "AggView layout changed: exported trees would no longer import");
 
 // What the C ABI and the renderer need from an aggregate: batches of closest-hit / any-hit
 // queries, with the batch size on the host or in device memory.
@@ -101,7 +103,6 @@ class DeviceAggregate : public RayTracer {
         bool used = false;
         void* last_stream = nullptr;
         int n_sms = 0;
-        void* window_stream = (void*)-1;  // the stream that last received the L2 access-policy window
     };
     int ensure_workspace(Workspace& w, uint64_t n, std::string* err) const;
     template <bool ANY>
@@ -111,8 +112,6 @@ class DeviceAggregate : public RayTracer {
     mutable std::mutex ws_mutex_;
     bool sort_rays_ = true;
     int stack_levels_ = 2;
-    size_t l2_window_bytes_ = 0;  // persisting L2 window over the nodes (0 = off)
-    float l2_hit_ratio_ = 1.0f;
     AggView view_{};
     AggregateStats stats_{};
     void* d_nodes_ = nullptr;

@@ -27,7 +27,6 @@
 #include "scene_json.hpp"
 #include "stratified.cuh"
 #include "surface.hpp"
-#include "tri_screen.h"
 #include "rrt_test.h"
 
 namespace {
@@ -1245,21 +1244,6 @@ int rrt_rays_f32_host_probe(uint64_t n_rays, const rrt_ray_f32* rays, rrt_ray* p
         return fail(RRT_ERR_INVALID, "rrt_rays_f32_host_probe: null argument");
     for (uint64_t i = 0; i < n_rays; ++i) promoted[i] = rrt::promote_ray(rays[i]);
     for (uint64_t i = 0; i < n_hits; ++i) compact[i] = rrt::compact_hit(hits[i]);
-    return RRT_OK;
-}
-
-int rrt_tri_screen_host_probe(uint64_t n, const double* o3, const double* d3, const double* best_t, const float* verts9,
-                              uint8_t* out) {
-    if (!o3 || !d3 || !best_t || !verts9 || !out) return fail(RRT_ERR_INVALID, "rrt_tri_screen_host_probe: null argument");
-    for (uint64_t i = 0; i < n; ++i) {
-        rrt::ScreenRay R = rrt::make_screen_ray(o3[3 * i], o3[3 * i + 1], o3[3 * i + 2], d3[3 * i], d3[3 * i + 1], d3[3 * i + 2]);
-        float bt = (float)best_t[i];  // __double2float_ru
-        if ((double)bt < best_t[i]) bt = std::nextafterf(bt, INFINITY);
-        R.bt = bt;
-        const float* v = verts9 + 9 * i;
-        // the PrimRec48 lanes: v0.xyz v1.x | v1.yz v2.xy | v2.z prim_id kind pad
-        out[i] = rrt::tri_surely_missed(R, rrt::V4f{v[0], v[1], v[2], v[3]}, rrt::V4f{v[4], v[5], v[6], v[7]}, rrt::V4f{v[8], 0.f, 0.f, 0.f}) ? 1 : 0;
-    }
     return RRT_OK;
 }
 
