@@ -145,9 +145,36 @@ int rrt_scene_commit(rrt_scene* scene, uint32_t max_prims_in_node, uint32_t buil
  * [first_instance, first_instance + n) — numbered in the order the rrt_scene_add_* calls appended them — and brings the
  * aggregate up to date: the moved primitives are re-baked to world space and the tree is made anew ON the device
  * (Morton keys, radix sort, radix tree, bottom-up boxes: milliseconds).  Fast tier; integrators made over the scene
- * must be destroyed first, since they hold its tables.                                                              */
+ * must be destroyed first, since they hold its tables.  Host-synchronous: it returns when the new aggregate is in
+ * place, and no other call on the scene may be in flight while it runs.                                           */
 int rrt_scene_update_instances(rrt_scene* scene, uint32_t first_instance, uint32_t n, const double* instance_m,
                                const double* instance_minv);
+/* New vertex positions p[3*n_vertices] for vertices [first_vertex, first_vertex + n_vertices) of mesh `mesh_id`, and
+ * optionally new vertex normals n[3*n_normals] for normals [first_normal, first_normal + n_normals).  Topology (vi, ni),
+ * uv and every instance transform stay.  Every primitive made from the mesh, bare or under any instance, moves.
+ * Afterwards every call on the scene answers as a fresh scene given the new vertices and committed with
+ * RRT_BUILD_DEVICE_LBVH would, and rrt_scene_export_tree returns that scene's bytes but for the two timing fields; a
+ * scene committed RRT_BUILD_FAST is an RRT_BUILD_DEVICE_LBVH scene afterwards (rrt_scene_build_info).
+ * How: the first update after a commit (or after rrt_scene_update_instances) bakes every primitive to world space and
+ * keeps that image in device memory: about 128 B per primitive, plus 24 B per vertex and 12 B per triangle of every
+ * mesh (1 Mi triangles: about 170 MB), plus the device tree builder's scratch, about 130 B per primitive, which a
+ * commit frees and an update keeps; all of it is freed by rrt_scene_destroy.  An update copies its range there,
+ * re-bakes the mesh's primitives on the device, takes the world box and node format by device reductions, builds the
+ * tree on the device and gathers the primitive records there.  Scenes for which a device commit builds the host SAH
+ * tree (16 primitives or fewer, one leaf, or a radix tree deeper than the traversal stack) get that tree here too.
+ * Errors leave the scene as it was: RRT_ERR_INVALID for a null pointer with a non-zero count, an unknown mesh, a vertex
+ * or normal range past the end, normals for a mesh without normals, an uncommitted scene, or live integrators over the
+ * scene; RRT_ERR_UNSUPPORTED in the literal tier.  Zero counts: RRT_OK, nothing rebuilt.
+ * Host-synchronous: it returns when the new aggregate is in place, and no other call on the scene may be in flight
+ * while it runs.                                                                                                   */
+int rrt_scene_update_mesh(rrt_scene* scene, uint32_t mesh_id, uint32_t first_vertex, uint32_t n_vertices, const double* p,
+                          uint32_t first_normal, uint32_t n_normals, const double* n);
+/* The same with DEVICE buffers, read in stream order on `cuda_stream` (after the work already queued there); the
+ * positions are copied into the image on the device, and both ranges are also brought into the scene's host copy of
+ * the mesh, which later commits, exports, instance updates and renderers read.                                     */
+int rrt_scene_update_mesh_device(rrt_scene* scene, uint32_t mesh_id, uint32_t first_vertex, uint32_t n_vertices,
+                                 const double* d_p, uint32_t first_normal, uint32_t n_normals, const double* d_n,
+                                 void* cuda_stream);
 int rrt_scene_num_prims(const rrt_scene* scene, uint32_t* out);
 /* Primitive::world_bound (bvh.rs:177-182): out6 = p_min, p_max.                                 */
 int rrt_world_bound(const rrt_scene* scene, double out6[6]);

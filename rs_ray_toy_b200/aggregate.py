@@ -197,6 +197,25 @@ class GpuAggregate:
         capi.check(self.L.rrt_scene_update_instances(self.h, first, m.shape[0], _ptr(m), _ptr(inv)))
         return self
 
+    def update_mesh(self, mesh: int, p, first_vertex: int = 0, normals=None, first_normal: int = 0):
+        """rrt_scene_update_mesh: new positions p[k, 3] for vertices [first_vertex, first_vertex + k) of `mesh` (and new
+        normals for [first_normal, ...) when given); every primitive made from the mesh moves.  Afterwards the scene
+        answers like a fresh one committed with RRT_BUILD_DEVICE_LBVH over the new geometry."""
+        p = np.ascontiguousarray(p, dtype=np.float64).reshape(-1, 3)
+        n = None if normals is None else np.ascontiguousarray(normals, dtype=np.float64).reshape(-1, 3)
+        capi.check(self.L.rrt_scene_update_mesh(self.h, mesh, first_vertex, p.shape[0], _ptr(p), first_normal,
+                                                0 if n is None else n.shape[0], _ptr(n)))
+        return self
+
+    def update_mesh_device(self, mesh: int, first_vertex: int, n_vertices: int, d_p: int, first_normal: int = 0,
+                           n_normals: int = 0, d_n: int = 0, stream: int = 0):
+        """rrt_scene_update_mesh_device: the same from device buffers (raw pointers, e.g. a float64 CUDA tensor's
+        data_ptr()), read after the work already queued on `stream`; returns when the new aggregate is in place."""
+        capi.check(self.L.rrt_scene_update_mesh_device(self.h, mesh, first_vertex, n_vertices, C.c_void_p(d_p or None),
+                                                       first_normal, n_normals, C.c_void_p(d_n or None),
+                                                       C.c_void_p(stream or None)))
+        return self
+
     def export_tree(self) -> np.ndarray:
         """rrt_scene_export_tree: the committed aggregate (tree + records + tables) as one uint8 blob."""
         n = C.c_uint64()

@@ -85,6 +85,8 @@ def lib() -> C.CDLL:
         "rrt_intersect_surface": (i32, [vp, u64, vp, vp]),
         "rrt_rays_f32_host_probe": (i32, [u64, vp, vp, u64, vp, vp]),
         "rrt_scene_update_instances": (i32, [vp, u32, u32, vp, vp]),
+        "rrt_scene_update_mesh": (i32, [vp, u32, u32, u32, vp, u32, u32, vp]),
+        "rrt_scene_update_mesh_device": (i32, [vp, u32, u32, u32, vp, u32, u32, vp, vp]),
         "rrt_scene_export_tree": (i32, [vp, vp, u64, C.POINTER(u64)]),
         "rrt_scene_commit_from_tree": (i32, [vp, vp, u64]),
     }

@@ -27,7 +27,10 @@
 #include "bvh_lbvh.hpp"
 #include "bvh_pack_plan.hpp"
 #include "device_layout.h"
+#include "bake_core.h"
+#include "mesh_update.hpp"
 #include "sphere_core.cuh"
+#include "world_bake.hpp"
 
 namespace rrt {
 
@@ -807,10 +810,26 @@ void parallel_ranges(size_t n, F f) {
     for (auto& th : pool) th.join();
 }
 
-bool fp32_exact(const double* v, int n) {
-    for (int i = 0; i < n; ++i)
-        if ((double)(float)v[i] != v[i]) return false;
-    return true;
+// Node32 when the grid costs the primitive boxes little (see DeviceAggregate::build): `growth` is the sum over the
+// primitive boxes of min(1, grid_cells / half-perimeter).  RRT_QUANTISE overrides.
+bool quantise_for(double growth, size_t n) {
+    bool quantise = RRT_NODE32 == 2;
+    if (RRT_NODE32 == 1) quantise = growth / (double)n < 0.05;
+    if (const char* e = std::getenv("RRT_QUANTISE")) quantise = atoi(e) != 0;
+    return quantise;
+}
+double grid_cells(const float grid_ext[3]) {
+    return 2.0 * ((double)grid_ext[0] + (double)grid_ext[1] + (double)grid_ext[2]) / 32768.0;
+}
+
+// The device builder makes ONE-primitive leaves whatever max_prims_in_node says (Tier-F answers do not depend on
+// it): without SAH the collapsed 2-4 primitive leaves cost more f64 tests than they save nodes — measured 1364
+// (1) / 1261 (2) / 1076 (4) Mrays/s on config 3 (profiles/r1_bench_build_lbvh.txt).  RRT_LBVH_LEAF overrides.
+uint32_t lbvh_leaf_for(uint32_t max_prims_in_node) {
+    const uint32_t max_leaf = max_prims_in_node == 0 ? 4 : (max_prims_in_node > 8 ? 8 : max_prims_in_node);
+    uint32_t lbvh_leaf = 1;
+    if (const char* e = std::getenv("RRT_LBVH_LEAF")) lbvh_leaf = (uint32_t)std::max(1, std::min(8, atoi(e)));
+    return std::min(max_leaf, lbvh_leaf);
 }
 
 #define RRT_CUDA(call)                                                                  \
@@ -824,69 +843,35 @@ bool fp32_exact(const double* v, int n) {
 
 }  // namespace
 
-DeviceAggregate::~DeviceAggregate() {
-    if (d_nodes_) cudaFree(d_nodes_);
-    if (d_prims_) cudaFree(d_prims_);
-    if (d_inst_) cudaFree(d_inst_);
-    if (d_gspheres_) cudaFree(d_gspheres_);
-    for (auto& kv : ws_) {
-        Workspace& w = kv.second;
-        if (w.d_bins) cudaFree(w.d_bins);
-        if (w.d_block_sums) cudaFree(w.d_block_sums);
-        if (w.d_small) cudaFree(w.d_small);
-        if (w.d_key) cudaFree(w.d_key);
-        if (w.d_rank) cudaFree(w.d_rank);
-        if (w.d_perm) cudaFree(w.d_perm);
-        if (w.last_use) cudaEventDestroy(w.last_use);
-    }
-}
-
-int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prims_in_node, std::string* err, bool device_lbvh) {
-    auto t_start = std::chrono::steady_clock::now();
-    const bool timing = std::getenv("RRT_BUILD_TIMING") != nullptr;
-    auto lap = [&, t_last = t_start](const char* what) mutable {
-        if (!timing) return;
-        auto now = std::chrono::steady_clock::now();
-        fprintf(stderr, "RRT_BUILD_TIMING %-22s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(now - t_last).count());
-        t_last = now;
-    };
-    device_ = device;
+int bake_world(const HostScene& scene, WorldBake* out, std::string* err) {
     const size_t n = scene.prims.size();
-    if (n == 0) {
-        if (err) *err = "BVHAccel::new needs at least one primitive (bvh.rs:319)";
-        return RRT_ERR_EMPTY;
-    }
-    if (n >= (1u << 28)) {
-        if (err) *err = "too many primitives for the 28-bit leaf reference";
-        return RRT_ERR_UNSUPPORTED;
-    }
-    // ---- bake to world space ----
-    struct World {
-        double v[9];
-    };
+    BakedPrim* const world = out->world.get();
+    Aabb* const boxes = out->boxes.get();
+    uint8_t* const kind = out->kind.get();
+    uint8_t* const exact = out->exact.get();
     // (default-initialised buffers: the worker threads below touch — and so place — their own pages; a value-initialised
     // std::vector would zero half a gigabyte on one thread first: measured 170 -> see profiles/r2_build_timing.txt)
-    RawBuf<World> world(n);
-    RawBuf<Aabb> boxes_buf(n);
-    Aabb* const boxes = boxes_buf.get();
     std::atomic<int> not_fp32{0}, clipped_with_own_transform{0};
-    RawBuf<uint8_t> general(n);  // spheres that need the object-space test (sphere_core.cuh)
     parallel_ranges(n, [&](size_t i0, size_t i1) {
     bool all_fp32 = true;
     for (size_t i = i0; i < i1; ++i) {
         const Primitive& pr = scene.prims[i];
         new (&boxes[i]) Aabb();
-        general[i] = 0;
+        exact[i] = 1;
         if (pr.kind == SHAPE_TRIANGLE) {
+            kind[i] = PRIM_TRIANGLE;
             scene.world_triangle(i, world[i].v);
-            for (int k = 0; k < 3; ++k) boxes[i].grow(&world[i].v[3 * k]);
-            if (all_fp32 && !fp32_exact(world[i].v, 9)) all_fp32 = false;
+            bake::triangle_box(world[i].v, boxes[i].lo, boxes[i].hi);
+            exact[i] = bake::fp32_exact(world[i].v, 9) ? 1 : 0;
+            if (!exact[i]) all_fp32 = false;
         } else {
+            for (int k = 0; k < 9; ++k) world[i].v[k] = 0.0;  // a PrimRec96 copies all nine
+            kind[i] = PRIM_SPHERE;
             const Sphere& s = scene.spheres[pr.shape];
             auto general_sphere = [&]() {
                 // box of the object-space extent [-r, r]^2 x [z_min, z_max] (Sphere::object_bound, sphere.rs:262-268)
                 // carried to world space corner by corner; the GenSphere entry itself is made after this loop
-                general[i] = 1;
+                kind[i] = PRIM_SPHERE_GENERAL;
                 const double zl = std::fmax(std::fmin(s.z_min, s.z_max), -s.radius), zh = std::fmin(std::fmax(s.z_min, s.z_max), s.radius);
                 for (int k = 0; k < 8; ++k) {
                     Vec3d q = s.obj_to_world.point(Vec3d{(k & 1) ? s.radius : -s.radius, (k & 2) ? s.radius : -s.radius, (k & 4) ? zh : zl});
@@ -952,9 +937,9 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
                    "its own: the reference clips the first root in instance space (Q5a) and its answer then depends on the tree";
         return RRT_ERR_UNSUPPORTED;
     }
-    std::vector<GenSphere> gspheres;
+    out->gspheres.clear();
     for (size_t i = 0; i < n; ++i) {
-        if (!general[i]) continue;
+        if (kind[i] != PRIM_SPHERE_GENERAL) continue;
         const Primitive& pr = scene.prims[i];
         const Sphere& s = scene.spheres[pr.shape];
         GenSphere g{};
@@ -971,11 +956,70 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
         g.theta_min = std::acos(std::fmin(std::fmax(std::fmin(s.z_min, s.z_max) / s.radius, -1.0), 1.0));
         g.theta_max = std::acos(std::fmin(std::fmax(std::fmax(s.z_min, s.z_max) / s.radius, -1.0), 1.0));
         g.clip.phi_max = std::fmin(std::fmax(s.phi_max_deg, 0.0), 360.0) * (kPiD / 180.0);
-        world[i].v[0] = (double)gspheres.size();
+        world[i].v[0] = (double)out->gspheres.size();
         world[i].v[3] = s.radius;
-        gspheres.push_back(g);
+        out->gspheres.push_back(g);
     }
-    const bool all_fp32 = not_fp32 == 0;
+    out->all_fp32 = not_fp32 == 0;
+    out->has_spheres = false;
+    for (const Primitive& pr : scene.prims) out->has_spheres |= pr.kind == SHAPE_SPHERE;
+    out->inst_w2p.clear();
+    if (out->has_spheres && !scene.instances.empty()) {
+        out->inst_w2p.resize(12 * scene.instances.size());
+        for (size_t i = 0; i < scene.instances.size(); ++i)
+            for (int r = 0; r < 3; ++r)
+                for (int c = 0; c < 4; ++c) out->inst_w2p[12 * i + 4 * r + c] = scene.instances[i].inv.m[r][c];
+    }
+    return RRT_OK;
+}
+
+bool DeviceAggregate::device_tree_fits(size_t n, uint32_t max_prims_in_node) {
+    const uint32_t max_leaf = max_prims_in_node == 0 ? 4 : (max_prims_in_node > 8 ? 8 : max_prims_in_node);
+    return n > 16 && n > max_leaf;
+}
+
+DeviceAggregate::~DeviceAggregate() {
+    if (d_nodes_) cudaFree(d_nodes_);
+    if (d_prims_) cudaFree(d_prims_);
+    if (d_inst_) cudaFree(d_inst_);
+    if (d_gspheres_) cudaFree(d_gspheres_);
+    for (auto& kv : ws_) {
+        Workspace& w = kv.second;
+        if (w.d_bins) cudaFree(w.d_bins);
+        if (w.d_block_sums) cudaFree(w.d_block_sums);
+        if (w.d_small) cudaFree(w.d_small);
+        if (w.d_key) cudaFree(w.d_key);
+        if (w.d_rank) cudaFree(w.d_rank);
+        if (w.d_perm) cudaFree(w.d_perm);
+        if (w.last_use) cudaEventDestroy(w.last_use);
+    }
+}
+
+int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prims_in_node, std::string* err, bool device_lbvh) {
+    auto t_start = std::chrono::steady_clock::now();
+    const bool timing = std::getenv("RRT_BUILD_TIMING") != nullptr;
+    auto lap = [&, t_last = t_start](const char* what) mutable {
+        if (!timing) return;
+        auto now = std::chrono::steady_clock::now();
+        fprintf(stderr, "RRT_BUILD_TIMING %-22s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(now - t_last).count());
+        t_last = now;
+    };
+    device_ = device;
+    const size_t n = scene.prims.size();
+    if (n == 0) {
+        if (err) *err = "BVHAccel::new needs at least one primitive (bvh.rs:319)";
+        return RRT_ERR_EMPTY;
+    }
+    if (n >= (1u << 28)) {
+        if (err) *err = "too many primitives for the 28-bit leaf reference";
+        return RRT_ERR_UNSUPPORTED;
+    }
+    // ---- bake to world space ----
+    WorldBake bake(n);
+    if (int rc = bake_world(scene, &bake, err)) return rc;
+    const BakedPrim* const world = bake.world.get();
+    Aabb* const boxes = bake.boxes.get();
+    const bool all_fp32 = bake.all_fp32;
     lap("bake to world space");
     // ---- frame: world box, fp32 margin, Node32 grid, node format ----
     Aabb world_box;
@@ -989,19 +1033,17 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
         });
     }
     const NodeFrame frame = make_node_frame(world_box);
-    const double scale = frame.scale, delta = frame.delta;
+    const double delta = frame.delta;
     const double* grid_lo = frame.grid_lo;
-    const double* grid_c = frame.grid_c;
     const float* grid_ext = frame.grid_ext;
     // The grid costs every box up to one cell per side.  That is nothing for a scene whose primitives are much
     // larger than extent / 32768 (configs 1-5: under 1% of a primitive box's half-perimeter), and it would ruin
     // the culling of a scene with small details in a huge box; such scenes keep the fp32 node.
-    bool quantise = RRT_NODE32 == 2;
+    double growth = 0.0;
     if (RRT_NODE32 == 1) {
-        const double cells = 2.0 * ((double)grid_ext[0] + (double)grid_ext[1] + (double)grid_ext[2]) / 32768.0;
+        const double cells = grid_cells(grid_ext);
         // (summed per contiguous range, then over the ranges in order: the same total whatever the thread count is not
         // guaranteed to the last bit, and does not need to be — it is compared with 5 %)
-        double growth = 0.0;
         std::mutex m;
         parallel_ranges(n, [&](size_t i0, size_t i1) {
             double part = 0.0;
@@ -1012,16 +1054,9 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
             std::lock_guard<std::mutex> lock(m);
             growth += part;
         });
-        quantise = growth / (double)n < 0.05;
     }
-    if (const char* e = std::getenv("RRT_QUANTISE")) quantise = atoi(e) != 0;
-    const uint32_t max_leaf = max_prims_in_node == 0 ? 4 : (max_prims_in_node > 8 ? 8 : max_prims_in_node);
-    const bool on_device = device_lbvh && n > 16 && n > max_leaf;
-    // The device builder makes ONE-primitive leaves whatever max_prims_in_node says (Tier-F answers do not depend on
-    // it): without SAH the collapsed 2-4 primitive leaves cost more f64 tests than they save nodes — measured 1364
-    // (1) / 1261 (2) / 1076 (4) Mrays/s on config 3 (profiles/r1_bench_build_lbvh.txt).  RRT_LBVH_LEAF overrides.
-    uint32_t lbvh_leaf = 1;
-    if (const char* e = std::getenv("RRT_LBVH_LEAF")) lbvh_leaf = (uint32_t)std::max(1, std::min(8, atoi(e)));
+    const bool quantise = quantise_for(growth, n);
+    const bool on_device = device_lbvh && device_tree_fits(n, max_prims_in_node);
 
     lap("frame + node format");
     // ---- tree ----
@@ -1029,7 +1064,7 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
     LbvhResult lb;
     bool on_device_ok = on_device;
     if (on_device) {
-        int rc = build_lbvh_device(device, AabbSpan(boxes, n), std::min(max_leaf, lbvh_leaf), delta, quantise, grid_lo, grid_ext, &lb, err);
+        int rc = build_lbvh_device(device, AabbSpan(boxes, n), lbvh_leaf_for(max_prims_in_node), delta, quantise, grid_lo, grid_ext, &lb, err);
         if (rc != RRT_OK) return rc;
         tree.max_depth = lb.max_depth + 1;
         tree.n_leaves = lb.n_leaves;
@@ -1056,7 +1091,7 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
             all_tri = all_tri && is_tri[i];
         }
         SplitTriangles tris;
-        tris.verts = world.get()->v;  // (World is nine doubles: primitive i's vertices start at 9 i)
+        tris.verts = world->v;  // (BakedPrim is nine doubles: primitive i's vertices start at 9 i)
         tris.is_tri = all_tri ? nullptr : is_tri.get();
         build_sah(AabbSpan(boxes, n), tris, sp, &tree);
         if (tree.max_depth + 2 > (uint32_t)kStack) {
@@ -1091,7 +1126,7 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
                 std::memset(&r, 0, sizeof(r));
                 std::memcpy(r.v, world[pi].v, sizeof(double) * 9);
                 r.prim_id = pi;
-                r.kind = pr.kind == SHAPE_TRIANGLE ? PRIM_TRIANGLE : (general[pi] ? PRIM_SPHERE_GENERAL : PRIM_SPHERE);
+                r.kind = bake.kind[pi];
                 r.pad[0] = pr.instance >= 0 ? (uint32_t)pr.instance : 0xFFFFFFFFu;
                 rec96[slot] = r;
             } else {
@@ -1109,7 +1144,7 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
                     for (int j = 0; j < 3; ++j) r.sph.c[j] = world[pi].v[j];
                     r.sph.radius = world[pi].v[3];
                     r.sph.prim_id = pi;
-                    r.sph.kind = general[pi] ? PRIM_SPHERE_GENERAL : PRIM_SPHERE;
+                    r.sph.kind = bake.kind[pi];
                     r.sph.instance = pr.instance >= 0 ? (uint32_t)pr.instance : 0xFFFFFFFFu;
                 }
                 rec48[slot] = r;
@@ -1230,58 +1265,140 @@ int DeviceAggregate::build(int device, const HostScene& scene, uint32_t max_prim
     RRT_CUDA(cudaMalloc(&d_prims_, prim_bytes));
     RRT_CUDA(cudaMemcpy(d_prims_, wide ? (const void*)rec96.get() : (const void*)rec48.get(), prim_bytes,
                         cudaMemcpyHostToDevice));
-    bool has_spheres = false;
-    for (const Primitive& pr : scene.prims) has_spheres |= pr.kind == SHAPE_SPHERE;
-    if (has_spheres && !scene.instances.empty()) {
-        std::vector<double> w2p(12 * scene.instances.size());
-        for (size_t i = 0; i < scene.instances.size(); ++i)
-            for (int r = 0; r < 3; ++r)
-                for (int c = 0; c < 4; ++c) w2p[12 * i + 4 * r + c] = scene.instances[i].inv.m[r][c];
-        RRT_CUDA(cudaMalloc(&d_inst_, w2p.size() * sizeof(double)));
-        RRT_CUDA(cudaMemcpy(d_inst_, w2p.data(), w2p.size() * sizeof(double), cudaMemcpyHostToDevice));
+    if (int rc = upload_tables(bake.inst_w2p, bake.gspheres, err)) return rc;
+    lap("upload");
+    Built b;
+    b.world_box = world_box;
+    b.frame = frame;
+    b.quantise = quantise;
+    b.wide = wide;
+    b.has_spheres = bake.has_spheres;
+    b.n_nodes = on_device_ok ? lb.n_nodes : nodes.size();
+    b.tree_device_usec = on_device_ok ? (uint64_t)(lb.device_ms * 1000.0f) : 0;
+    b.n_leaves = tree.n_leaves;
+    b.max_depth = tree.max_depth;
+    b.node_bytes = node_bytes;
+    b.prim_bytes = prim_bytes;
+    b.n_records = n_refs;
+    b.n_prims = n;
+    install(b, t_start);
+    return RRT_OK;
+}
+
+int DeviceAggregate::build_from_image(int device, MeshImage& image, uint32_t max_prims_in_node, bool* too_deep,
+                                      std::string* err) {
+    const auto t_start = std::chrono::steady_clock::now();
+    const bool timing = std::getenv("RRT_BUILD_TIMING") != nullptr;
+    auto lap = [&, t_last = t_start](const char* what) mutable {
+        if (!timing) return;
+        auto now = std::chrono::steady_clock::now();
+        fprintf(stderr, "RRT_BUILD_TIMING %-22s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(now - t_last).count());
+        t_last = now;
+    };
+    *too_deep = false;
+    device_ = device;
+    RRT_CUDA(cudaSetDevice(device));
+    const size_t n = image.n_prims();
+    // ---- frame: world box (device min / max, then make_node_frame on its 48 bytes), node format ----
+    Aabb world_box;
+    bool all_fp32 = true;
+    if (int rc = image.frame(&world_box, &all_fp32, err)) return rc;
+    const NodeFrame frame = make_node_frame(world_box);
+    // The growth sum is a parallel sum on the device, rounded differently from the host's: only a scene within rounding
+    // of the 5 % threshold can get the other node format than a fresh commit.
+    double growth = 0.0;
+    if (RRT_NODE32 == 1)
+        if (int rc = image.growth(grid_cells(frame.grid_ext), &growth, err)) return rc;
+    const bool quantise = quantise_for(growth, n);
+    lap("frame + node format");
+    // ---- tree ----
+    LbvhResult lb;
+    if (int rc = build_lbvh_device_boxes(device, image.boxes(), (uint32_t)n, lbvh_leaf_for(max_prims_in_node), frame.delta,
+                                         quantise, frame.grid_lo, frame.grid_ext, &image.arena(), &lb, err))
+        return rc;
+    if (lb.max_depth + 1 + 2 > (uint32_t)kStack) {
+        cudaFree(lb.d_nodes);
+        *too_deep = true;
+        return RRT_OK;
+    }
+    d_nodes_ = lb.d_nodes;
+    lap("device LBVH (total)");
+    // ---- records in tree order, tables ----
+    const bool wide = !all_fp32;
+    const size_t prim_bytes = n * (wide ? sizeof(PrimRec96) : sizeof(PrimRec48));
+    RRT_CUDA(cudaMalloc(&d_prims_, prim_bytes));
+    if (int rc = image.gather(lb.d_order, wide, d_prims_, err)) return rc;
+    if (int rc = upload_tables(image.inst_w2p, image.gspheres, err)) return rc;
+    RRT_CUDA(cudaStreamSynchronize(0));
+    lap("records + tables");
+    Built b;
+    b.world_box = world_box;
+    b.frame = frame;
+    b.quantise = quantise;
+    b.wide = wide;
+    b.has_spheres = image.has_spheres;
+    b.n_nodes = lb.n_nodes;
+    b.tree_device_usec = (uint64_t)(lb.device_ms * 1000.0f);
+    b.n_leaves = lb.n_leaves;
+    b.max_depth = lb.max_depth + 1;
+    b.node_bytes = lb.node_bytes;
+    b.prim_bytes = prim_bytes;
+    b.n_records = n;
+    b.n_prims = n;
+    install(b, t_start);
+    return RRT_OK;
+}
+
+int DeviceAggregate::upload_tables(const std::vector<double>& inst_w2p, const std::vector<GenSphere>& gspheres, std::string* err) {
+    if (!inst_w2p.empty()) {
+        RRT_CUDA(cudaMalloc(&d_inst_, inst_w2p.size() * sizeof(double)));
+        RRT_CUDA(cudaMemcpy(d_inst_, inst_w2p.data(), inst_w2p.size() * sizeof(double), cudaMemcpyHostToDevice));
     }
     if (!gspheres.empty()) {
         RRT_CUDA(cudaMalloc(&d_gspheres_, gspheres.size() * sizeof(GenSphere)));
         RRT_CUDA(cudaMemcpy(d_gspheres_, gspheres.data(), gspheres.size() * sizeof(GenSphere), cudaMemcpyHostToDevice));
     }
+    inst_bytes_ = inst_w2p.size() * sizeof(double);
+    gsphere_bytes_ = gspheres.size() * sizeof(GenSphere);
+    return RRT_OK;
+}
+
+// The view, statistics and launch set-up of a built aggregate whose nodes, records and tables are on the device.
+void DeviceAggregate::install(const Built& b, std::chrono::steady_clock::time_point t_start) {
     view_.gspheres = d_gspheres_;
-    lap("upload");
     view_.inst_w2p = static_cast<const double*>(d_inst_);
-    view_.has_spheres = has_spheres ? 1 : 0;
+    view_.has_spheres = b.has_spheres ? 1 : 0;
     view_.nodes = d_nodes_;
     view_.prims = d_prims_;
     for (int k = 0; k < 3; ++k) {
-        view_.world_lo[k] = world_box.lo[k] - delta;
-        view_.world_hi[k] = world_box.hi[k] + delta;
+        view_.world_lo[k] = b.world_box.lo[k] - b.frame.delta;
+        view_.world_hi[k] = b.world_box.hi[k] + b.frame.delta;
     }
-    view_.scene_scale = scale;
+    view_.scene_scale = b.frame.scale;
     for (int k = 0; k < 3; ++k) {
-        view_.grid_c[k] = grid_c[k];
-        view_.grid_ext[k] = grid_ext[k];
+        view_.grid_c[k] = b.frame.grid_c[k];
+        view_.grid_ext[k] = b.frame.grid_ext[k];
     }
-    view_.quantised = quantise ? 1 : 0;
+    view_.quantised = b.quantise ? 1 : 0;
     view_.root = 0;
-    view_.wide = wide ? 1 : 0;
+    view_.wide = b.wide ? 1 : 0;
     view_.sort_mode = 0;
     if (const char* e = std::getenv("RRT_SORT_MODE")) view_.sort_mode = atoi(e);
     if (const char* e = std::getenv("RRT_SORT")) sort_rays_ = atoi(e) != 0;
-    stats_.n_nodes = on_device_ok ? lb.n_nodes : nodes.size();
-    stats_.tree_device_usec = on_device_ok ? (uint64_t)(lb.device_ms * 1000.0f) : 0;
-    stats_.n_leaves = tree.n_leaves;
-    stats_.max_depth = tree.max_depth;
-    stats_.device_bytes = node_bytes + prim_bytes;
-    stats_.n_records = n_refs;
-    stats_.wide_records = wide;
-    stats_.n_prims = n;
+    stats_.n_nodes = b.n_nodes;
+    stats_.tree_device_usec = b.tree_device_usec;
+    stats_.n_leaves = b.n_leaves;
+    stats_.max_depth = b.max_depth;
+    stats_.device_bytes = b.node_bytes + b.prim_bytes;
+    stats_.n_records = b.n_records;
+    stats_.wide_records = b.wide;
+    stats_.n_prims = b.n_prims;
     stats_.build_usec =
         (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t_start).count();
-    stack_levels_ = (int)tree.max_depth + 2;
-    node_bytes_ = node_bytes;
-    prim_bytes_ = prim_bytes;
-    inst_bytes_ = d_inst_ ? 12 * scene.instances.size() * sizeof(double) : 0;
-    gsphere_bytes_ = gspheres.size() * sizeof(GenSphere);
-    configure_kernels(quantise);
-    return RRT_OK;
+    stack_levels_ = (int)b.max_depth + 2;
+    node_bytes_ = b.node_bytes;
+    prim_bytes_ = b.prim_bytes;
+    configure_kernels(b.quantise);
 }
 
 // the only shared memory is the traversal stack (one entry per tree level + the marker, trace_smem_bytes);
@@ -1292,7 +1409,9 @@ void DeviceAggregate::configure_kernels(bool quantise) {
     if (carve > 100) carve = 100;
     for (int v = 0; v < 16; ++v) {
         const void* fn = (const void*)trace_kernel_for(v & 1, v & 2, v & 4, v & 8);
-        cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        // (the attribute belongs to the kernel, shared by every aggregate in the process: it is set to what the deepest
+        // tree needs, so that configuring a shallower aggregate never refuses a deeper one's launch)
+        cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)trace_smem_bytes(kStack));
         cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
     }
 }

@@ -2,16 +2,22 @@
 // closest-hit / any-hit kernels.  Host-visible part (no CUDA types in the interface besides
 // the opaque stream pointer) so capi.cpp can be compiled by the plain host compiler.
 #pragma once
+#include <chrono>
 #include <cstdint>
 #include <map>
 #include <mutex>
 #include <string>
+#include <vector>
 
 #include "../../include/rrt.h"
+#include "bvh_lbvh.hpp"
 #include "bvh_sah.hpp"
 #include "host_scene.hpp"
 
 namespace rrt {
+
+struct GenSphere;
+class MeshImage;
 
 struct AggregateStats {
     uint64_t n_nodes = 0, n_leaves = 0, max_depth = 0, device_bytes = 0, build_usec = 0, n_records = 0,
@@ -68,6 +74,14 @@ class DeviceAggregate : public RayTracer {
     // Returns an rrt_status; on failure *err holds the reason.
     // `device_lbvh`: build the tree on the GPU (bvh_lbvh.cu) instead of the host SAH builder.
     int build(int device, const HostScene& scene, uint32_t max_prims_in_node, std::string* err, bool device_lbvh = false);
+    // Whether build(device_lbvh = true) makes the tree on the device for n primitives: more than 16, and more than one
+    // leaf holds.  Otherwise it builds the host SAH tree.
+    static bool device_tree_fits(size_t n, uint32_t max_prims_in_node);
+    // The aggregate build(device_lbvh = true) makes, from a scene baked on the device (rrt_scene_update_mesh): world box,
+    // node format, device LBVH and records, without the primitives going through the host.  For n that
+    // device_tree_fits.  *too_deep: the radix tree is deeper than the traversal stack; nothing was built, and build()
+    // (which falls back to the SAH tree) is the caller's answer.
+    int build_from_image(int device, MeshImage& image, uint32_t max_prims_in_node, bool* too_deep, std::string* err);
 
     // Asynchronous on `stream`; *launches (optional) receives the number of kernels launched.
     int closest_hit(uint64_t n, const rrt_ray* d_rays, rrt_hit* d_hits, void* stream, std::string* err,
@@ -121,6 +135,14 @@ class DeviceAggregate : public RayTracer {
     uint64_t node_bytes_ = 0, prim_bytes_ = 0, inst_bytes_ = 0, gsphere_bytes_ = 0;
     int device_ = 0;
     void configure_kernels(bool quantised);
+    int upload_tables(const std::vector<double>& inst_w2p, const std::vector<GenSphere>& gspheres, std::string* err);
+    struct Built {
+        Aabb world_box;
+        NodeFrame frame;
+        bool quantise, wide, has_spheres;
+        uint64_t n_nodes, n_leaves, max_depth, tree_device_usec, node_bytes, prim_bytes, n_records, n_prims;
+    };
+    void install(const Built& b, std::chrono::steady_clock::time_point t_start);
 };
 
 }  // namespace rrt

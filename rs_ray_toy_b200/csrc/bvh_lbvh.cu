@@ -16,6 +16,7 @@
 
 #include "bvh_lbvh.hpp"
 #include "lbvh_core.h"
+#include "reduce.cuh"
 
 namespace rrt {
 
@@ -266,16 +267,197 @@ __global__ void __launch_bounds__(256) depth_kernel(uint32_t n, const RadixNode*
 
 }  // namespace
 
+namespace {
+
+struct Lap {
+    bool on = std::getenv("RRT_BUILD_TIMING") != nullptr;
+    std::chrono::steady_clock::time_point last = std::chrono::steady_clock::now();
+    void operator()(const char* what) {
+        if (!on) return;
+        const auto now = std::chrono::steady_clock::now();
+        fprintf(stderr, "RRT_BUILD_TIMING   lbvh: %-18s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(now - last).count());
+        last = now;
+    }
+};
+
+// Every scratch array of a build over n primitives in ONE allocation (15 cudaMalloc + 15 cudaFree cost 30-80 ms).
+struct ArenaLayout {
+    size_t o_boxes, o_leaf_box, o_node_box, o_keys, o_keys_sorted, o_vals, o_order, o_visits, o_keep, o_new, o_out2, o_nodes,
+        o_pnode, o_pleaf, o_tmp, hist_words, total = 0;
+    explicit ArenaLayout(uint32_t n) {
+        const uint32_t ni = n - 1;
+        const uint32_t sort_tiles = (n + kSortTile - 1) / kSortTile;
+        hist_words = 256 * (size_t)sort_tiles;
+        const size_t scratch_words = std::max(scan_scratch_words(hist_words), scan_scratch_words(ni));
+        o_boxes = reserve((size_t)n * sizeof(BoxF));
+        o_leaf_box = reserve((size_t)n * sizeof(BoxF));
+        o_node_box = reserve((size_t)ni * sizeof(BoxF));
+        o_keys = reserve((size_t)n * sizeof(uint64_t));
+        o_keys_sorted = reserve((size_t)n * sizeof(uint64_t));
+        o_vals = reserve((size_t)n * sizeof(uint32_t));
+        o_order = reserve((size_t)n * sizeof(uint32_t));
+        o_visits = reserve((size_t)ni * sizeof(uint32_t));
+        o_keep = reserve((size_t)ni * sizeof(uint32_t));
+        o_new = reserve((size_t)ni * sizeof(uint32_t));
+        o_out2 = reserve(2 * sizeof(uint32_t));
+        o_nodes = reserve((size_t)ni * sizeof(RadixNode));
+        o_pnode = reserve((size_t)ni * sizeof(int32_t));
+        o_pleaf = reserve((size_t)n * sizeof(int32_t));
+        o_tmp = reserve((hist_words + scratch_words) * sizeof(uint32_t));
+    }
+    size_t reserve(size_t bytes) {
+        const size_t at = total;
+        total += (bytes + 255) & ~(size_t)255;
+        return at;
+    }
+};
+
+// The build from the fp32 boxes already in the arena (layout ArenaLayout(n)) and their centroid frame: keys, sort,
+// hierarchy, boxes, collapse, emitted nodes.  out->d_order points into the arena.
+int build_in_arena(uint32_t n, char* d_arena, const CentroidFrame& fr, uint32_t max_leaf, double delta, bool quantise,
+                   const double grid_lo[3], const float grid_ext[3], LbvhResult* out, std::string* err, Lap& lap) {
+    const ArenaLayout L(n);
+    EmitParams P;
+    P.max_leaf = max_leaf;
+    P.quantise = quantise ? 1 : 0;
+    P.delta = delta;
+    for (int k = 0; k < 3; ++k) {
+        P.grid_lo[k] = grid_lo[k];
+        P.grid_ext[k] = (double)grid_ext[k];
+    }
+    BoxF* d_boxes = reinterpret_cast<BoxF*>(d_arena + L.o_boxes);
+    BoxF* d_leaf_box = reinterpret_cast<BoxF*>(d_arena + L.o_leaf_box);
+    BoxF* d_node_box = reinterpret_cast<BoxF*>(d_arena + L.o_node_box);
+    uint64_t* d_keys = reinterpret_cast<uint64_t*>(d_arena + L.o_keys);
+    uint64_t* d_keys_sorted = reinterpret_cast<uint64_t*>(d_arena + L.o_keys_sorted);
+    uint32_t* d_vals = reinterpret_cast<uint32_t*>(d_arena + L.o_vals);
+    uint32_t* d_order = reinterpret_cast<uint32_t*>(d_arena + L.o_order);
+    uint32_t* d_visits = reinterpret_cast<uint32_t*>(d_arena + L.o_visits);
+    uint32_t* d_keep = reinterpret_cast<uint32_t*>(d_arena + L.o_keep);
+    uint32_t* d_new = reinterpret_cast<uint32_t*>(d_arena + L.o_new);
+    uint32_t* d_out2 = reinterpret_cast<uint32_t*>(d_arena + L.o_out2);
+    RadixNode* d_nodes = reinterpret_cast<RadixNode*>(d_arena + L.o_nodes);
+    int32_t* d_pnode = reinterpret_cast<int32_t*>(d_arena + L.o_pnode);
+    int32_t* d_pleaf = reinterpret_cast<int32_t*>(d_arena + L.o_pleaf);
+    void* d_tmp = d_arena + L.o_tmp;
+    void* d_emit = nullptr;
+#define LB_TRY(call)                                                            \
+    do {                                                                        \
+        cudaError_t e_ = (call);                                                \
+        if (e_ != cudaSuccess) {                                                \
+            if (err) *err = std::string(#call) + ": " + cudaGetErrorString(e_); \
+            if (d_emit) cudaFree(d_emit);                                       \
+            return RRT_ERR_CUDA;                                                \
+        }                                                                       \
+    } while (0)
+    const uint32_t ni = n - 1;
+    LB_TRY(cudaMemset(d_visits, 0, (size_t)ni * sizeof(uint32_t)));
+    LB_TRY(cudaMemset(d_out2, 0, 2 * sizeof(uint32_t)));
+
+    cudaEvent_t e0, e1;
+    LB_TRY(cudaEventCreate(&e0));
+    LB_TRY(cudaEventCreate(&e1));
+    LB_TRY(cudaEventRecord(e0, 0));
+    const unsigned gb = (n + 255) / 256, gi = (ni + 255) / 256;
+    keys_kernel<<<gb, 256>>>(n, d_boxes, fr, d_keys, d_vals);
+    uint32_t* d_hist = static_cast<uint32_t*>(d_tmp);
+    uint32_t* d_scan_scratch = d_hist + L.hist_words;
+    // 63-bit Morton keys: eight 8-bit passes (an even number: the sorted pairs end where they started, then swap names)
+    if (radix_sort_pairs(d_keys, d_vals, d_keys_sorted, d_order, n, 64, d_hist, d_scan_scratch, 0) == 0) {
+        std::swap(d_keys, d_keys_sorted);
+        std::swap(d_vals, d_order);
+    }
+    hierarchy_kernel<<<gi, 256>>>(n, d_keys_sorted, d_nodes, d_pnode, d_pleaf);
+    refit_kernel<<<gb, 256>>>(n, d_boxes, d_order, d_nodes, d_pnode, d_pleaf, d_leaf_box, d_node_box, d_visits);
+    flag_kernel<<<gi, 256>>>(ni, d_nodes, max_leaf, d_keep);
+    exclusive_scan_u32(d_keep, d_new, ni, d_scan_scratch, 0);
+    uint32_t last_keep = 0, last_new = 0;
+    LB_TRY(cudaMemcpy(&last_keep, d_keep + (ni - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    LB_TRY(cudaMemcpy(&last_new, d_new + (ni - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    const uint32_t n_kept = last_new + last_keep;
+    const size_t node_size = quantise ? sizeof(Node32) : sizeof(Node64);
+    LB_TRY(cudaMalloc(&d_emit, (size_t)n_kept * node_size));
+    if (quantise) emit_kernel<true><<<gi, 256>>>(ni, d_nodes, d_keep, d_new, d_leaf_box, d_node_box, P, d_emit);
+    else emit_kernel<false><<<gi, 256>>>(ni, d_nodes, d_keep, d_new, d_leaf_box, d_node_box, P, d_emit);
+    depth_kernel<<<gb, 256>>>(n, d_nodes, d_keep, d_pnode, d_pleaf, d_out2);
+    LB_TRY(cudaEventRecord(e1, 0));
+    LB_TRY(cudaGetLastError());
+    LB_TRY(cudaEventSynchronize(e1));
+    float ms = 0.0f;
+    cudaEventElapsedTime(&ms, e0, e1);
+    cudaEventDestroy(e0);
+    cudaEventDestroy(e1);
+    lap("kernels");
+    uint32_t out2[2] = {0, 0};
+    LB_TRY(cudaMemcpy(out2, d_out2, sizeof(out2), cudaMemcpyDeviceToHost));
+    // the root's box (for the caller's world bound): node 0 of the radix tree
+    BoxF root;
+    LB_TRY(cudaMemcpy(&root, d_node_box, sizeof(BoxF), cudaMemcpyDeviceToHost));
+    for (int k = 0; k < 3; ++k) {
+        out->root_lo[k] = root.lo[k];
+        out->root_hi[k] = root.hi[k];
+    }
+    out->d_order = d_order;
+    out->d_nodes = d_emit;
+    out->node_bytes = (size_t)n_kept * node_size;
+    out->n_nodes = n_kept;
+    out->max_depth = out2[0];
+    out->n_leaves = out2[1];
+    out->device_ms = ms;
+    return RRT_OK;
+#undef LB_TRY
+}
+
+CentroidFrame centroid_frame(const double clo[3], const double chi[3]) {
+    CentroidFrame fr;
+    for (int k = 0; k < 3; ++k) {
+        fr.lo[k] = down_f(clo[k]);
+        const double ext = chi[k] - (double)fr.lo[k];
+        fr.inv_ext[k] = ext > 0.0 ? (float)(1.0 / ext) : 0.0f;
+    }
+    return fr;
+}
+
+// f64 boxes -> fp32 boxes rounded outward (the host conversion's down_f / up_f), and the bounds of their centroids:
+// a min / max, so the same values whatever order the blocks fold in.
+struct CentroidBounds {
+    double lo[3], hi[3];
+};
+__global__ void __launch_bounds__(256) boxes_f32_kernel(uint32_t n, const Aabb* __restrict__ boxes, BoxF* __restrict__ out,
+                                                         CentroidBounds* __restrict__ cb) {
+    double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        BoxF f;
+        for (int k = 0; k < 3; ++k) {
+            f.lo[k] = down_f(boxes[i].lo[k]);
+            f.hi[k] = up_f(boxes[i].hi[k]);
+            const double c = 0.5 * (double)f.lo[k] + 0.5 * (double)f.hi[k];
+            lo[k] = fmin(lo[k], c);
+            hi[k] = fmax(hi[k], c);
+        }
+        out[i] = f;
+    }
+    for (int k = 0; k < 3; ++k) {
+        lo[k] = warp_min_f64(lo[k]);
+        hi[k] = warp_max_f64(hi[k]);
+    }
+    if ((threadIdx.x & 31u) == 0)
+        for (int k = 0; k < 3; ++k) {
+            atomic_min_f64(&cb->lo[k], lo[k]);
+            atomic_max_f64(&cb->hi[k], hi[k]);
+        }
+}
+
+}  // namespace
+
+LbvhArena::~LbvhArena() {
+    if (d) cudaFree(d);
+}
+
 int build_lbvh_device(int device, AabbSpan boxes, uint32_t max_leaf, double delta, bool quantise,
                       const double grid_lo[3], const float grid_ext[3], LbvhResult* out, std::string* err) {
     const auto t0 = std::chrono::steady_clock::now();
-    const bool timing = std::getenv("RRT_BUILD_TIMING") != nullptr;
-    auto lap = [&, t_last = t0](const char* what) mutable {
-        if (!timing) return;
-        const auto now = std::chrono::steady_clock::now();
-        fprintf(stderr, "RRT_BUILD_TIMING   lbvh: %-18s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(now - t_last).count());
-        t_last = now;
-    };
+    Lap lap;
     const uint32_t n = (uint32_t)boxes.size();
     if (n < 2 || n <= max_leaf) {
         if (err) *err = "device LBVH needs more primitives than one leaf holds";
@@ -313,141 +495,69 @@ int build_lbvh_device(int device, AabbSpan boxes, uint32_t max_leaf, double delt
             }
     }
     lap("fp32 boxes (host)");
-    CentroidFrame fr;
-    for (int k = 0; k < 3; ++k) {
-        fr.lo[k] = down_f(clo[k]);
-        const double ext = chi[k] - (double)fr.lo[k];
-        fr.inv_ext[k] = ext > 0.0 ? (float)(1.0 / ext) : 0.0f;
-    }
-    EmitParams P;
-    P.max_leaf = max_leaf;
-    P.quantise = quantise ? 1 : 0;
-    P.delta = delta;
-    for (int k = 0; k < 3; ++k) {
-        P.grid_lo[k] = grid_lo[k];
-        P.grid_ext[k] = (double)grid_ext[k];
-    }
-
-    BoxF *d_boxes = nullptr, *d_leaf_box = nullptr, *d_node_box = nullptr;
-    uint64_t *d_keys = nullptr, *d_keys_sorted = nullptr;
-    uint32_t *d_vals = nullptr, *d_order = nullptr, *d_visits = nullptr, *d_keep = nullptr, *d_new = nullptr, *d_out2 = nullptr;
-    RadixNode* d_nodes = nullptr;
-    int32_t *d_pnode = nullptr, *d_pleaf = nullptr;
-    void *d_tmp = nullptr, *d_emit = nullptr;
-    char* d_arena = nullptr;  // every scratch array of the build: ONE allocation (15 cudaMalloc + 15 cudaFree cost 30-80 ms)
-    auto cleanup = [&]() {
-        if (d_arena) cudaFree(d_arena);
-        d_arena = nullptr;
-    };
-#define LB_TRY(call)                                                            \
-    do {                                                                        \
-        cudaError_t e_ = (call);                                                \
-        if (e_ != cudaSuccess) {                                                \
-            if (err) *err = std::string(#call) + ": " + cudaGetErrorString(e_); \
-            cleanup();                                                          \
-            if (d_emit) cudaFree(d_emit);                                       \
-            return RRT_ERR_CUDA;                                                \
-        }                                                                       \
-    } while (0)
-    const uint32_t ni = n - 1;
-    const uint32_t sort_tiles = (n + kSortTile - 1) / kSortTile;
-    const size_t hist_words = 256 * (size_t)sort_tiles;
-    const size_t scratch_words = std::max(scan_scratch_words(hist_words), scan_scratch_words(ni));
-    {
-        size_t total = 0;
-        auto reserve = [&](size_t bytes) {
-            const size_t at = total;
-            total += (bytes + 255) & ~(size_t)255;
-            return at;
-        };
-        const size_t o_boxes = reserve((size_t)n * sizeof(BoxF)), o_leaf_box = reserve((size_t)n * sizeof(BoxF)),
-                     o_node_box = reserve((size_t)ni * sizeof(BoxF)), o_keys = reserve((size_t)n * sizeof(uint64_t)),
-                     o_keys_sorted = reserve((size_t)n * sizeof(uint64_t)), o_vals = reserve((size_t)n * sizeof(uint32_t)),
-                     o_order = reserve((size_t)n * sizeof(uint32_t)), o_visits = reserve((size_t)ni * sizeof(uint32_t)),
-                     o_keep = reserve((size_t)ni * sizeof(uint32_t)), o_new = reserve((size_t)ni * sizeof(uint32_t)),
-                     o_out2 = reserve(2 * sizeof(uint32_t)), o_nodes = reserve((size_t)ni * sizeof(RadixNode)),
-                     o_pnode = reserve((size_t)ni * sizeof(int32_t)), o_pleaf = reserve((size_t)n * sizeof(int32_t)),
-                     o_tmp = reserve((hist_words + scratch_words) * sizeof(uint32_t));
-        LB_TRY(cudaMalloc(&d_arena, total));
-        d_boxes = reinterpret_cast<BoxF*>(d_arena + o_boxes);
-        d_leaf_box = reinterpret_cast<BoxF*>(d_arena + o_leaf_box);
-        d_node_box = reinterpret_cast<BoxF*>(d_arena + o_node_box);
-        d_keys = reinterpret_cast<uint64_t*>(d_arena + o_keys);
-        d_keys_sorted = reinterpret_cast<uint64_t*>(d_arena + o_keys_sorted);
-        d_vals = reinterpret_cast<uint32_t*>(d_arena + o_vals);
-        d_order = reinterpret_cast<uint32_t*>(d_arena + o_order);
-        d_visits = reinterpret_cast<uint32_t*>(d_arena + o_visits);
-        d_keep = reinterpret_cast<uint32_t*>(d_arena + o_keep);
-        d_new = reinterpret_cast<uint32_t*>(d_arena + o_new);
-        d_out2 = reinterpret_cast<uint32_t*>(d_arena + o_out2);
-        d_nodes = reinterpret_cast<RadixNode*>(d_arena + o_nodes);
-        d_pnode = reinterpret_cast<int32_t*>(d_arena + o_pnode);
-        d_pleaf = reinterpret_cast<int32_t*>(d_arena + o_pleaf);
-        d_tmp = d_arena + o_tmp;
-    }
+    const CentroidFrame fr = centroid_frame(clo, chi);
+    const ArenaLayout L(n);
+    char* d_arena = nullptr;
+    LB_CUDA(cudaMalloc(&d_arena, L.total));
     lap("cudaMalloc (arena)");
-    LB_TRY(cudaMemcpy(d_boxes, hb.get(), (size_t)n * sizeof(BoxF), cudaMemcpyHostToDevice));
+    int rc = RRT_OK;
+    cudaError_t e = cudaMemcpy(d_arena + L.o_boxes, hb.get(), (size_t)n * sizeof(BoxF), cudaMemcpyHostToDevice);
     lap("boxes H2D");
-    LB_TRY(cudaMemset(d_visits, 0, (size_t)ni * sizeof(uint32_t)));
-    LB_TRY(cudaMemset(d_out2, 0, 2 * sizeof(uint32_t)));
-
-    cudaEvent_t e0, e1;
-    LB_TRY(cudaEventCreate(&e0));
-    LB_TRY(cudaEventCreate(&e1));
-    LB_TRY(cudaEventRecord(e0, 0));
-    const unsigned gb = (n + 255) / 256, gi = (ni + 255) / 256;
-    keys_kernel<<<gb, 256>>>(n, d_boxes, fr, d_keys, d_vals);
-    uint32_t* d_hist = static_cast<uint32_t*>(d_tmp);
-    uint32_t* d_scan_scratch = d_hist + hist_words;
-    // 63-bit Morton keys: eight 8-bit passes (an even number: the sorted pairs end where they started, then swap names)
-    if (radix_sort_pairs(d_keys, d_vals, d_keys_sorted, d_order, n, 64, d_hist, d_scan_scratch, 0) == 0) {
-        std::swap(d_keys, d_keys_sorted);
-        std::swap(d_vals, d_order);
+    if (e != cudaSuccess) {
+        if (err) *err = std::string("cudaMemcpy (boxes): ") + cudaGetErrorString(e);
+        rc = RRT_ERR_CUDA;
     }
-    hierarchy_kernel<<<gi, 256>>>(n, d_keys_sorted, d_nodes, d_pnode, d_pleaf);
-    refit_kernel<<<gb, 256>>>(n, d_boxes, d_order, d_nodes, d_pnode, d_pleaf, d_leaf_box, d_node_box, d_visits);
-    flag_kernel<<<gi, 256>>>(ni, d_nodes, max_leaf, d_keep);
-    exclusive_scan_u32(d_keep, d_new, ni, d_scan_scratch, 0);
-    uint32_t last_keep = 0, last_new = 0;
-    LB_TRY(cudaMemcpy(&last_keep, d_keep + (ni - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    LB_TRY(cudaMemcpy(&last_new, d_new + (ni - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    const uint32_t n_kept = last_new + last_keep;
-    const size_t node_size = quantise ? sizeof(Node32) : sizeof(Node64);
-    LB_TRY(cudaMalloc(&d_emit, (size_t)n_kept * node_size));
-    if (quantise) emit_kernel<true><<<gi, 256>>>(ni, d_nodes, d_keep, d_new, d_leaf_box, d_node_box, P, d_emit);
-    else emit_kernel<false><<<gi, 256>>>(ni, d_nodes, d_keep, d_new, d_leaf_box, d_node_box, P, d_emit);
-    depth_kernel<<<gb, 256>>>(n, d_nodes, d_keep, d_pnode, d_pleaf, d_out2);
-    LB_TRY(cudaEventRecord(e1, 0));
-    LB_TRY(cudaGetLastError());
-    LB_TRY(cudaEventSynchronize(e1));
-    float ms = 0.0f;
-    cudaEventElapsedTime(&ms, e0, e1);
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    lap("kernels");
-    uint32_t out2[2] = {0, 0};
-    LB_TRY(cudaMemcpy(out2, d_out2, sizeof(out2), cudaMemcpyDeviceToHost));
-    out->order.resize(n);
-    LB_TRY(cudaMemcpy(out->order.data(), d_order, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    // the root's box (for the caller's world bound): node 0 of the radix tree
-    BoxF root;
-    LB_TRY(cudaMemcpy(&root, d_node_box, sizeof(BoxF), cudaMemcpyDeviceToHost));
-    for (int k = 0; k < 3; ++k) {
-        out->root_lo[k] = root.lo[k];
-        out->root_hi[k] = root.hi[k];
+    if (rc == RRT_OK) rc = build_in_arena(n, d_arena, fr, max_leaf, delta, quantise, grid_lo, grid_ext, out, err, lap);
+    if (rc == RRT_OK) {
+        out->order.resize(n);
+        e = cudaMemcpy(out->order.data(), out->d_order, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost);
+        out->d_order = nullptr;
+        if (e != cudaSuccess) {
+            if (err) *err = std::string("cudaMemcpy (order): ") + cudaGetErrorString(e);
+            cudaFree(out->d_nodes);
+            out->d_nodes = nullptr;
+            rc = RRT_ERR_CUDA;
+        }
+        lap("order D2H");
     }
-    lap("order D2H");
-    cleanup();
+    cudaFree(d_arena);
     lap("cudaFree (arena)");
-    out->d_nodes = d_emit;
-    out->node_bytes = (size_t)n_kept * node_size;
-    out->n_nodes = n_kept;
-    out->max_depth = out2[0];
-    out->n_leaves = out2[1];
-    out->device_ms = ms;
     out->total_usec = (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t0).count();
-    return RRT_OK;
-#undef LB_TRY
+    return rc;
+}
+
+int build_lbvh_device_boxes(int device, const Aabb* d_boxes, uint32_t n, uint32_t max_leaf, double delta, bool quantise,
+                            const double grid_lo[3], const float grid_ext[3], LbvhArena* arena, LbvhResult* out,
+                            std::string* err) {
+    const auto t0 = std::chrono::steady_clock::now();
+    Lap lap;
+    if (n < 2 || n <= max_leaf) {
+        if (err) *err = "device LBVH needs more primitives than one leaf holds";
+        return RRT_ERR_UNSUPPORTED;
+    }
+    LB_CUDA(cudaSetDevice(device));
+    const ArenaLayout L(n);
+    // the arena also holds the centroid bounds, after the build's arrays
+    const size_t need = L.total + sizeof(CentroidBounds);
+    if (arena->bytes < need) {
+        if (arena->d) cudaFree(arena->d);
+        arena->d = nullptr;
+        arena->bytes = 0;
+        LB_CUDA(cudaMalloc(&arena->d, need));
+        arena->bytes = need;
+    }
+    char* d_arena = static_cast<char*>(arena->d);
+    CentroidBounds* d_cb = reinterpret_cast<CentroidBounds*>(d_arena + L.total);
+    const CentroidBounds init = {{INFINITY, INFINITY, INFINITY}, {-INFINITY, -INFINITY, -INFINITY}};
+    LB_CUDA(cudaMemcpy(d_cb, &init, sizeof(init), cudaMemcpyHostToDevice));
+    boxes_f32_kernel<<<std::min<uint32_t>((n + 255) / 256, 1024u), 256>>>(n, d_boxes, reinterpret_cast<BoxF*>(d_arena + L.o_boxes), d_cb);
+    LB_CUDA(cudaGetLastError());
+    CentroidBounds cb;
+    LB_CUDA(cudaMemcpy(&cb, d_cb, sizeof(cb), cudaMemcpyDeviceToHost));
+    lap("fp32 boxes (device)");
+    const int rc = build_in_arena(n, d_arena, centroid_frame(cb.lo, cb.hi), max_leaf, delta, quantise, grid_lo, grid_ext, out, err, lap);
+    out->total_usec = (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t0).count();
+    return rc;
 }
 
 // Host run of the same per-element code, for the CPU tests (a checker, not a product path): returns the emitted

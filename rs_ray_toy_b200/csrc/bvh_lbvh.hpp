@@ -43,13 +43,31 @@ struct LbvhResult {
     size_t node_bytes = 0;
     uint32_t n_nodes = 0, n_leaves = 0, max_depth = 0;
     std::vector<uint32_t> order;  // primitive index at every sorted position (= record order)
+    const uint32_t* d_order = nullptr;  // build_lbvh_device_boxes: the same order in device memory, in the arena
     double root_lo[3], root_hi[3];
     float device_ms = 0.0f;       // keys -> emitted nodes, CUDA events
     uint64_t total_usec = 0;      // including allocations and transfers
 };
 
+// Device memory the builds over device boxes reuse: the scratch arrays, grown to the largest build, freed with it.
+struct LbvhArena {
+    void* d = nullptr;
+    size_t bytes = 0;
+    LbvhArena() = default;
+    LbvhArena(const LbvhArena&) = delete;
+    LbvhArena& operator=(const LbvhArena&) = delete;
+    ~LbvhArena();
+};
+
 int build_lbvh_device(int device, AabbSpan boxes, uint32_t max_leaf, double delta, bool quantise,
                       const double grid_lo[3], const float grid_ext[3], LbvhResult* out, std::string* err);
+
+// The same build from f64 boxes already in device memory (d_boxes[n]): the fp32 conversion and the centroid frame are
+// made on the device, the scratch lives in *arena, and the order stays there (out->d_order, valid until the arena's
+// next build; out->order is left empty).
+int build_lbvh_device_boxes(int device, const Aabb* d_boxes, uint32_t n, uint32_t max_leaf, double delta, bool quantise,
+                            const double grid_lo[3], const float grid_ext[3], LbvhArena* arena, LbvhResult* out,
+                            std::string* err);
 
 int lbvh_host_probe(const std::vector<Aabb>& boxes, uint32_t max_leaf, double delta, bool quantise, const double grid_lo[3],
                     const float grid_ext[3], std::vector<uint8_t>* nodes_out, std::vector<uint32_t>* order_out, uint32_t* depth_out,

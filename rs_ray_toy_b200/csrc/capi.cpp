@@ -20,6 +20,7 @@
 #include "bvh_hlbvh.hpp"
 #include "halton.cuh"
 #include "literal.hpp"
+#include "mesh_update.hpp"
 #include "png_min.hpp"
 #include "rays_f32.cuh"
 #include "rays_f32.hpp"
@@ -172,6 +173,10 @@ struct rrt_scene {
     // aggregate's own
     mutable std::mutex surface_mutex;
     mutable rrt::SurfaceTables* surface_tables = nullptr;
+
+    // the primitives baked on the device, made by the first rrt_scene_update_mesh after a commit, dropped by
+    // rrt_scene_update_instances (its runs hold the instance transforms)
+    std::unique_ptr<rrt::MeshImage> mesh_image;
 
     ~rrt_scene() {
         for (auto& kv : scratch) {
@@ -614,6 +619,7 @@ int rrt_scene_update_instances(rrt_scene* scene, uint32_t first_instance, uint32
     try {
         for (uint32_t i = 0; i < n; ++i)
             scene->host.instances[first_instance + i] = xf_from(instance_m + 16 * (size_t)i, instance_minv + 16 * (size_t)i);
+        scene->mesh_image.reset();
         // The tree over the moved primitives is made anew on the device: keys, sort, hierarchy and boxes take a few
         // milliseconds there (DESIGN.md §4b) — a topology-preserving refit would save none of the part that costs, the
         // host-side re-bake of the moved primitives' records.
@@ -632,6 +638,123 @@ int rrt_scene_update_instances(rrt_scene* scene, uint32_t first_instance, uint32
         return fail(RRT_ERR_INVALID, e.what());
     }
     return RRT_OK;
+}
+
+namespace {
+
+// rrt_scene_update_mesh and rrt_scene_update_mesh_device: d_stream is the caller's stream for device buffers, or
+// nullptr for host buffers.
+int update_mesh(rrt_scene* scene, const char* name, uint32_t mesh_id, uint32_t first_vertex, uint32_t n_vertices,
+                const double* p, uint32_t first_normal, uint32_t n_normals, const double* nrm, bool device,
+                cudaStream_t stream) {
+    const std::string fn = name;
+    if (!scene || (n_vertices && !p) || (n_normals && !nrm)) return fail(RRT_ERR_INVALID, fn + ": null argument");
+    if (!scene->committed) return fail(RRT_ERR_INVALID, fn + ": scene is not committed");
+    if (scene->build_flags == RRT_BUILD_LITERAL)
+        return fail(RRT_ERR_UNSUPPORTED, fn + ": the literal tier rebuilds the reference's HLBVH on the host; commit a new scene");
+    if (scene->live_renders.load() != 0)
+        return fail(RRT_ERR_INVALID, fn + ": destroy the integrators made over this scene first (they hold its tables)");
+    if (mesh_id >= scene->host.meshes.size()) return fail(RRT_ERR_INVALID, fn + ": bad mesh id");
+    rrt::TriangleMesh& mesh = scene->host.meshes[mesh_id];
+    if ((uint64_t)first_vertex + n_vertices > mesh.p.size() / 3) return fail(RRT_ERR_INVALID, fn + ": vertex range out of bounds");
+    if (n_normals && mesh.n.empty()) return fail(RRT_ERR_INVALID, fn + ": the mesh has no vertex normals");
+    if ((uint64_t)first_normal + n_normals > mesh.n.size() / 3) return fail(RRT_ERR_INVALID, fn + ": normal range out of bounds");
+    if (n_vertices == 0 && n_normals == 0) return RRT_OK;
+    try {
+        std::string err;
+        const int dev = scene->ctx->device;
+        CAPI_CUDA(cudaSetDevice(dev));
+        // a fresh RRT_BUILD_DEVICE_LBVH commit builds its tree on the device only for scenes that device_tree_fits;
+        // the others get the host SAH tree, and so does the update
+        const bool on_device = rrt::DeviceAggregate::device_tree_fits(scene->host.prims.size(), scene->max_prims_in_node);
+        if (on_device && !scene->mesh_image) {
+            std::unique_ptr<rrt::MeshImage> image(new rrt::MeshImage());
+            int rc = image->create(dev, scene->host, &err);
+            if (rc != RRT_OK) return fail(rc, err);
+            scene->mesh_image = std::move(image);
+        }
+        rrt::MeshImage* image = on_device ? scene->mesh_image.get() : nullptr;
+        const size_t p_bytes = 3 * (size_t)n_vertices * sizeof(double), n_bytes = 3 * (size_t)n_normals * sizeof(double);
+        double* const mp = mesh.p.data() + 3 * (size_t)first_vertex;
+        double* const mn = mesh.n.data() + 3 * (size_t)first_normal;
+        // The host mirror (later commits, exports, instance updates, renderers and the surface tables read it) takes the
+        // new values once the aggregate over them exists; the device entry reads the caller's buffers in stream order.
+        auto write_mirror = [&]() -> cudaError_t {
+            if (!device) {
+                if (n_vertices) std::memcpy(mp, p, p_bytes);
+                if (n_normals) std::memcpy(mn, nrm, n_bytes);
+                return cudaSuccess;
+            }
+            cudaError_t e = cudaSuccess;
+            if (n_vertices) e = cudaMemcpyAsync(mp, p, p_bytes, cudaMemcpyDeviceToHost, stream);
+            if (e == cudaSuccess && n_normals) e = cudaMemcpyAsync(mn, nrm, n_bytes, cudaMemcpyDeviceToHost, stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+            return e;
+        };
+        std::unique_ptr<rrt::DeviceAggregate> fresh(new rrt::DeviceAggregate());
+        bool built = false;
+        if (image) {
+            // the new positions into the image, then re-bake, frame, tree and records on the device
+            int rc = RRT_OK;
+            cudaError_t e = cudaSuccess;
+            double* const ip = image->positions(mesh_id) + 3 * (size_t)first_vertex;
+            if (n_vertices && device) {
+                e = cudaMemcpyAsync(ip, p, p_bytes, cudaMemcpyDeviceToDevice, stream);
+                if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+            } else if (n_vertices) {
+                e = cudaMemcpy(ip, p, p_bytes, cudaMemcpyHostToDevice);
+            }
+            if (e != cudaSuccess) rc = cuda_fail("the new positions to the device", e);
+            bool too_deep = false;
+            if (rc == RRT_OK && (rc = image->rebake(mesh_id, &err)) != RRT_OK) fail(rc, err);
+            if (rc == RRT_OK && (rc = fresh->build_from_image(dev, *image, scene->max_prims_in_node, &too_deep, &err)) != RRT_OK)
+                fail(rc, err);
+            built = rc == RRT_OK && !too_deep;
+            if (built && (e = write_mirror()) != cudaSuccess) rc = cuda_fail("the new values to the host", e);
+            if (rc != RRT_OK) {
+                scene->mesh_image.reset();
+                return rc;
+            }
+        }
+        if (!built) {
+            // the host SAH tree of a commit (too few primitives, or thousands with one centroid), made from the mirror
+            const std::vector<double> old_p(mp, mp + 3 * (size_t)n_vertices), old_n(mn, mn + 3 * (size_t)n_normals);
+            const cudaError_t e = write_mirror();
+            int rc = e == cudaSuccess ? RRT_OK : cuda_fail("the new values to the host", e);
+            fresh.reset(new rrt::DeviceAggregate());
+            if (rc == RRT_OK && (rc = fresh->build(dev, scene->host, scene->max_prims_in_node, &err, true)) != RRT_OK) fail(rc, err);
+            if (rc != RRT_OK) {
+                if (n_vertices) std::memcpy(mp, old_p.data(), p_bytes);
+                if (n_normals) std::memcpy(mn, old_n.data(), n_bytes);
+                scene->mesh_image.reset();
+                return rc;
+            }
+        }
+        scene->agg = std::move(fresh);
+        scene->build_flags = RRT_BUILD_DEVICE_LBVH;
+        // the surface pass's tables hold the old positions and normals: the next surface call uploads them anew
+        std::lock_guard<std::mutex> lock(scene->surface_mutex);
+        rrt::surface_tables_destroy(scene->surface_tables);
+        scene->surface_tables = nullptr;
+    } catch (const std::exception& e) {
+        return fail(RRT_ERR_INVALID, e.what());
+    }
+    return RRT_OK;
+}
+
+}  // namespace
+
+int rrt_scene_update_mesh(rrt_scene* scene, uint32_t mesh_id, uint32_t first_vertex, uint32_t n_vertices, const double* p,
+                          uint32_t first_normal, uint32_t n_normals, const double* n) {
+    return update_mesh(scene, "rrt_scene_update_mesh", mesh_id, first_vertex, n_vertices, p, first_normal, n_normals, n,
+                       false, nullptr);
+}
+
+int rrt_scene_update_mesh_device(rrt_scene* scene, uint32_t mesh_id, uint32_t first_vertex, uint32_t n_vertices,
+                                 const double* d_p, uint32_t first_normal, uint32_t n_normals, const double* d_n,
+                                 void* cuda_stream) {
+    return update_mesh(scene, "rrt_scene_update_mesh_device", mesh_id, first_vertex, n_vertices, d_p, first_normal, n_normals,
+                       d_n, true, static_cast<cudaStream_t>(cuda_stream));
 }
 
 int rrt_scene_num_prims(const rrt_scene* scene, uint32_t* out) {

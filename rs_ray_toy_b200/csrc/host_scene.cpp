@@ -1,5 +1,7 @@
 #include "host_scene.hpp"
 
+#include "bake_core.h"
+
 namespace rrt {
 
 Transform Transform::identity() {
@@ -17,14 +19,9 @@ bool Transform::is_identity() const {
 }
 
 Vec3d Transform::point(Vec3d p) const {
-    const auto& a = m.m;
-    double xp = a[0][0] * p.x + a[0][1] * p.y + a[0][2] * p.z + a[0][3];
-    double yp = a[1][0] * p.x + a[1][1] * p.y + a[1][2] * p.z + a[1][3];
-    double zp = a[2][0] * p.x + a[2][1] * p.y + a[2][2] * p.z + a[2][3];
-    double wp = a[3][0] * p.x + a[3][1] * p.y + a[3][2] * p.z + a[3][3];
-    if (wp == 1.0) return {xp, yp, zp};
-    double inv_w = 1.0 / wp;
-    return {inv_w * xp, inv_w * yp, inv_w * zp};
+    double q[3];
+    bake::xf_point(&m.m[0][0], p.x, p.y, p.z, q);
+    return {q[0], q[1], q[2]};
 }
 
 Vec3d Transform::vector(Vec3d v) const {
@@ -42,14 +39,7 @@ Vec3d Transform::normal(Vec3d n) const {
 void HostScene::world_triangle(size_t i, double v[9]) const {
     const Primitive& pr = prims[i];
     const TriangleMesh& m = meshes[pr.shape];
-    for (int k = 0; k < 3; ++k) {
-        uint32_t vi = m.vi[3 * (size_t)pr.tri + k];
-        Vec3d p{m.p[3 * (size_t)vi], m.p[3 * (size_t)vi + 1], m.p[3 * (size_t)vi + 2]};
-        if (pr.instance >= 0) p = instances[pr.instance].point(p);
-        v[3 * k] = p.x;
-        v[3 * k + 1] = p.y;
-        v[3 * k + 2] = p.z;
-    }
+    bake::world_triangle(m.p.data(), m.vi.data(), pr.tri, pr.instance >= 0 ? &instances[pr.instance].m.m[0][0] : nullptr, v);
 }
 
 namespace {

@@ -128,6 +128,8 @@ extern "C" {
                                 instance_m: *const f64, instance_minv: *const f64) -> c_int;
     pub fn rrt_scene_commit(scene: *mut rrt_scene, max_prims_in_node: u32, build_flags: u32) -> c_int;
     pub fn rrt_scene_update_instances(scene: *mut rrt_scene, first_instance: u32, n: u32, instance_m: *const f64, instance_minv: *const f64) -> c_int;
+    pub fn rrt_scene_update_mesh(scene: *mut rrt_scene, mesh_id: u32, first_vertex: u32, n_vertices: u32, p: *const f64, first_normal: u32, n_normals: u32, n: *const f64) -> c_int;
+    pub fn rrt_scene_update_mesh_device(scene: *mut rrt_scene, mesh_id: u32, first_vertex: u32, n_vertices: u32, d_p: *const f64, first_normal: u32, n_normals: u32, d_n: *const f64, cuda_stream: *mut c_void) -> c_int;
     pub fn rrt_scene_num_prims(scene: *const rrt_scene, out: *mut u32) -> c_int;
     pub fn rrt_world_bound(scene: *const rrt_scene, out6: *mut f64) -> c_int;
     pub fn rrt_scene_export_tree(scene: *const rrt_scene, buffer: *mut c_void, capacity: u64, bytes: *mut u64) -> c_int;
